@@ -2,6 +2,7 @@
 """bench.py - NMPC solves/s of the fused closed-loop step (BASELINE.json metric) on N B200s, one process per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model force|jerk] [--batch B]
+                    [--dump-outputs DIR]
 
 A "step" is one control step for the whole batch of drones: yref windowing + x0 embedding + SQP/HPIPM solve + converter
 + plant step + logs (bnmpc_closed_loop_run).  Workload of the headline at every N: BASELINE config 2, "force_model
@@ -20,17 +21,25 @@ own 4096 instances, no data-path collective).
 
 --impl reference times the CPU restatement of the reference's path (oracle/nmpc_oracle.c, all host threads) - acados
 itself is not installable here (DESIGN.md) - on the same instances (same generator, same global ids), a bounded sample.
+
+--dump-outputs DIR writes what the timed closed loop returned for its last control step as DIR/<name>.npy (float64), so
+that two builds can be compared output for output; the inputs are seeded and identical from run to run.
+
+bench.py writes nothing into the source tree (which may be read-only): what it compiles at run time goes to a temporary
+directory.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True          # no __pycache__ in the tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -135,17 +144,16 @@ def workload(lo, hi, n_steps, rows, N, mass_sigma=0.0, with_noise=True):
 def native_oracle(model):
     """The C restatement rebuilt for THIS host (bench.py runs on the GPU box): -O3 -march=native with the model's dimensions
     as compile-time constants (ORC_FIXED_NX / NU), so the CPU baseline is the port at its best.  Timing only - the parity
-    tests use the generic build."""
+    tests use the generic build.  Built in a temporary directory, removed once the library is loaded."""
     from oracle import c_oracle as co
     nx, nu = (6, 2) if model == 'jerk' else (4, 2)
     src = os.path.join(ROOT, 'oracle', 'nmpc_oracle.c')
-    out = os.path.join(ROOT, 'oracle', '_build', f'libnmpc_oracle_native_{nx}_{nu}.so')
     flags = ['-O3', '-march=native', f'-DORC_FIXED_NX={nx}', f'-DORC_FIXED_NU={nu}']
     try:
-        if not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(src):
-            os.makedirs(os.path.dirname(out), exist_ok=True)
+        with tempfile.TemporaryDirectory(prefix='bnmpc_oracle_') as tmp:
+            out = os.path.join(tmp, f'libnmpc_oracle_native_{nx}_{nu}.so')
             subprocess.check_call(['gcc'] + flags + ['-pthread', '-fPIC', '-shared', '-o', out, src, '-lm'])
-        return co.load_variant(out), ' '.join(flags)
+            return co.load_variant(out), ' '.join(flags)
     except Exception as e:   # noqa: BLE001
         return co.lib(), f'generic build -O3 -mavx2 -mfma (native rebuild failed: {type(e).__name__})'
 
@@ -252,6 +260,8 @@ def run_ours(args):
     if world > 1:
         dist.all_reduce(stats)                    # the only collective of the headline: final per-step metrics (< 1 KB)
     qp_local = float(qp.sum())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res, S - 1, rank, world)
     del loop, res
 
     # ---- e2e: the reference's loop shape through the shim with pinned host buffers, every step ------------------------
@@ -333,6 +343,40 @@ def run_ours(args):
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_HEADER_BYTES = 1024        # room kept for the header of each .npy file
+
+
+def dump_outputs(out_dir, res, step, rank, world):
+    """--dump-outputs: what BatchedClosedLoop.results() gives a caller for control step `step` (the last timed one) - the
+    plant state after it, controller and plant inputs, carried acceleration, status and QP iterations - and the per-drone
+    totals of the run (closed-loop cost, AED, failed steps), one row per drone in global instance order, as float64 .npy.
+    Above DUMP_LIMIT_BYTES the rows are a fixed seeded sample of the drones; `drone.npy` holds the global ids of the rows."""
+    import torch
+    arrays = {'Xsim': res['Xsim'][:, step + 1], 'U_ctrl': res['U_ctrl'][:, step], 'U_plant': res['U_plant'][:, step],
+              'a': res['a'][:, step], 'status': res['status'][:, step], 'qp_iter': res['qp_iter'][:, step],
+              'cost': res['cost'], 'aed': res['aed'], 'failures': res['failures']}
+    arrays = {k: v.double().contiguous() for k, v in arrays.items()}
+    if world > 1:                                   # every rank owns the same number of drones (weak scaling), in rank order
+        import torch.distributed as dist
+        for k, v in arrays.items():
+            parts = [torch.empty_like(v) for _ in range(world)]
+            dist.all_gather(parts, v)
+            arrays[k] = torch.cat(parts)
+    if rank != 0:
+        return
+    total = arrays['cost'].shape[0]
+    row_bytes = 8 * (1 + sum(v[0].numel() for v in arrays.values()))
+    max_rows = (DUMP_LIMIT_BYTES - DUMP_HEADER_BYTES * (1 + len(arrays))) // row_bytes
+    rows = np.arange(total)
+    if total > max_rows:
+        rows = np.sort(np.random.default_rng(SEED).choice(total, max_rows, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'drone.npy'), rows.astype(np.float64))
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f'{k}.npy'), v.cpu().numpy()[rows])
 
 
 def run_e2e(args, pkg, dev, local, inp, ref_im, world, barrier, allmax, Ke):
@@ -662,7 +706,12 @@ def main():
     ap.add_argument('--e2e-groups', type=int, default=4, help='solver objects (streams) the e2e leg splits the batch into (SolverFleet)')
     ap.add_argument('--cpu-instances', type=int, default=4096)
     ap.add_argument('--cpu-steps', type=int, default=400, help='closed-loop steps of the cpu_baseline sample (~10-20 s of CPU work on 16 cores)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed control step as DIR/<name>.npy (float64)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs dumps the GPU path; the reference arm has no outputs to dump')
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == 'reference':
