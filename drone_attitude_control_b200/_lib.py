@@ -66,6 +66,8 @@ def lib():
         'bnmpc_set': (C.c_int, [vp, C.c_int, C.c_int, dp, C.c_int]),
         'bnmpc_get': (C.c_int, [vp, C.c_int, C.c_int, dp, C.c_int]),
         'bnmpc_set_yref_all': (C.c_int, [vp, dp, C.c_int]),
+        'bnmpc_set_ref_table': (C.c_int, [vp, dp, C.c_int, C.c_int, C.c_int, C.c_int]),
+        'bnmpc_set_yref_row': (C.c_int, [vp, C.c_int]),
         'bnmpc_reset': (C.c_int, [vp]),
         'bnmpc_solve': (C.c_int, [vp]),
         'bnmpc_get_stats': (C.c_int, [vp, C.c_int, vp, C.c_int]),

@@ -132,6 +132,36 @@ class BatchedAcadosOcpSolver:
         check(lib().bnmpc_set_yref_all(self._h, ptr, on_dev))
         self._keep_y = keep
 
+    def set_ref_table(self, table):
+        """Bind the whole reference trajectory once (bnmpc_set_ref_table): [rows, cols] shared by all drones or [batch, rows,
+        cols] one per drone, row r = [xref_r (nx) | uref_r (nu) | ignored] - the gen_circle_traj table (8 columns) of the
+        force / jerk models, the [xref | uref] table (14 columns) of the 3-D model.  torch (CUDA or CPU) or numpy; the
+        solver keeps its own copy.  None releases the binding.  Select a window with set_yref_row(i)."""
+        if table is None:
+            check(lib().bnmpc_set_ref_table(self._h, None, 0, 0, 0, 0))
+            return
+        if isinstance(table, torch.Tensor):
+            t = table.detach().to(torch.float64)
+        else:
+            t = torch.from_numpy(np.asarray(table, dtype=np.float64))
+        if t.dim() == 3 and t.shape[0] != self.batch:
+            raise ValueError(f'per-drone table: expected {self.batch} tables, got {t.shape[0]}')
+        if t.dim() not in (2, 3) or t.shape[-1] < self.nx + self.nu or t.shape[-2] < self.N + 1:
+            raise ValueError(f'expected a table [rows >= {self.N + 1}, cols >= {self.nx + self.nu}] or [{self.batch}, rows, cols], '
+                             f'got {tuple(t.shape)}')
+        if t.is_cuda and t.device != self.device:
+            t = t.to(self.device)
+        t = t.contiguous()
+        if t.is_cuda:
+            torch.cuda.current_stream(t.device).synchronize()       # the copy runs on the solver's stream
+        rows, cols = int(t.shape[-2]), int(t.shape[-1])
+        check(lib().bnmpc_set_ref_table(self._h, C.c_void_p(t.data_ptr()), rows, cols, 1 if t.dim() == 2 else 2, int(t.is_cuda)))
+
+    def set_yref_row(self, i):
+        """OCP.set_up_ocp(i, xref, uref) (src/force_model/ocp.py:117-122) on the table of set_ref_table: the solves read
+        yref_k = rows i + k of it, no upload.  set_yref_all() switches back to uploaded windows."""
+        check(lib().bnmpc_set_yref_row(self._h, int(i)))
+
     def solve(self):
         ev0 = torch.cuda.Event(enable_timing=True); ev1 = torch.cuda.Event(enable_timing=True)
         ev0.record(self._stream)

@@ -50,6 +50,10 @@ struct Handle {
     int ls_generation;             // BNMPC_LS_GENERATION: see LoopArgs::ls_generation
     long long* prof; int prof_cap; // bnmpc_debug_profile
     int64_t launches;
+    // reference table bound by bnmpc_set_ref_table ([rows][cols], or [batch][rows][cols] when not shared), FP64
+    double* tab; size_t tab_cap;   // device copy, its capacity in doubles
+    int tab_rows, tab_cols, tab_shared;
+    bool tab_sel; int tab_row;     // the table (window at tab_row) is the yref source of the solves, not Gs::YREF
 };
 
 const ModelOps* pick_ops(int model, int precision) {
@@ -151,6 +155,25 @@ __global__ void k_yref_all(const __grid_constant__ Gs<T> gs, int NX, int NU, int
     if (inst >= gs.B) return;
     const int k = e < gs.N * ny ? e / ny : gs.N, j = e - k * ny;
     *field_ptr(gs, NX, NU, NP, inst, F_YREF, k, j) = T(aos[idx]);
+}
+
+// the window of the bound table -> Gs::YREF, all stages (what bnmpc_set_yref_all of that window stores)
+template <class T>
+__global__ void k_yref_from_table(const __grid_constant__ Gs<T> gs, int NX, int NU, int NP, const __grid_constant__ ApiRef t) {
+    const int ny = NX + NU, per = gs.N * ny + NX;
+    const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int inst = (int)(idx / per), e = (int)(idx % per);
+    if (inst >= gs.B) return;
+    const int k = e < gs.N * ny ? e / ny : gs.N, j = e - k * ny;
+    *field_ptr(gs, NX, NU, NP, inst, F_YREF, k, j) = T(api_ref_row(t, inst, k)[j]);
+}
+// get(k, 'yref') from the bound table: the values the solve reads (rounded to T), AoS [B][dim]
+template <class T>
+__global__ void k_yref_table_get(int B, const __grid_constant__ ApiRef t, int k, int dim, double* aos) {
+    const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int inst = (int)(idx / dim), j = (int)(idx % dim);
+    if (inst >= B) return;
+    aos[idx] = double(T(api_ref_row(t, inst, k)[j]));
 }
 
 // p_ctrl [NP][B] batch-minor -> parameters
@@ -433,6 +456,25 @@ int bound_xfer(Handle* h, int field, int stage, double* aos, int to_state) {
     return 0;
 }
 
+// the yref source of the next solve: the bound table's window, or Gs::YREF
+ApiRef api_ref(const Handle* h) {
+    if (!h->tab_sel) return ApiRef{nullptr, 0, 0, 0, 0};
+    return ApiRef{h->tab, h->tab_rows, h->tab_cols, h->tab_shared, h->tab_row};
+}
+
+// selected table -> Gs::YREF (one gather kernel, converting to T), which is the yref source from then on
+int materialise_window(Handle* h) {
+    if (!h->tab_sel) return 0;
+    const ApiRef t = api_ref(h);
+    const size_t tot = ((size_t)h->cfg.horizon * (h->ops->nx + h->ops->nu) + h->ops->nx) * h->batch;
+    const unsigned grid = (unsigned)((tot + 127) / 128);
+    if (h->ops->elem_size == 8) k_yref_from_table<double><<<grid, 128, 0, h->stream>>>(gs_cast<double>(h->gs), h->ops->nx, h->ops->nu, h->ops->np, t);
+    else k_yref_from_table<float><<<grid, 128, 0, h->stream>>>(gs_cast<float>(h->gs), h->ops->nx, h->ops->nu, h->ops->np, t);
+    CK(cudaGetLastError()); h->launches++;
+    h->tab_sel = false;
+    return 0;
+}
+
 int reset_iterate(Handle* h) {
     const size_t es = h->ops->elem_size, B = h->batch;
     CK(cudaMemsetAsync(h->gs.V, 0, B * h->nV * es, h->stream));
@@ -631,6 +673,7 @@ int bnmpc_destroy(void* handle) {
     if (h->xs) cudaFree(h->xs);
     if (h->gs.U0) cudaFree(h->gs.U0);
     if (h->gs.BND) cudaFree(h->gs.BND);
+    if (h->tab) cudaFree(h->tab);
     for (int i = 0; i < 4; i++) if (h->stage[i]) cudaFree(h->stage[i]);
     if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -665,7 +708,7 @@ int bnmpc_dims(void* handle, int32_t dims[7]) {
 
 int64_t bnmpc_workspace_bytes(void* handle) {
     Handle* h = (Handle*)handle;
-    return h ? (int64_t)(h->gs_bytes + sizeof(int32_t) * 4 * h->batch + sizeof(double) * 11 * h->Bp) : 0;
+    return h ? (int64_t)(h->gs_bytes + sizeof(int32_t) * 4 * h->batch + sizeof(double) * 11 * h->Bp + sizeof(double) * h->tab_cap) : 0;
 }
 
 int bnmpc_set(void* handle, int stage, int field, const double* value, int on_device) {
@@ -682,6 +725,8 @@ int bnmpc_set(void* handle, int stage, int field, const double* value, int on_de
         if (int rc = ensure_bounds(h)) return rc;
         return bound_xfer(h, field, stage, const_cast<double*>(d), 1);
     }
+    if (field == F_YREF)           // one stage of the table's window: the whole window becomes the stored yref first
+        if (int rc = materialise_window(h)) return rc;
     CK(field_xfer(h, field, stage, const_cast<double*>(d), dim, dim, 1));
     return 0;
 }
@@ -700,6 +745,14 @@ int bnmpc_get(void* handle, int stage, int field, double* out, int on_device) {
         if (int rc = bound_xfer(h, field, stage, d, 0)) return rc;
         return stage_out_end(h, 1, out, (size_t)h->batch * dim, on_device);
     }
+    if (field == F_YREF && h->tab_sel) {           // read straight from the table: no handle state changes
+        const size_t tot = (size_t)h->batch * dim;
+        const unsigned grid = (unsigned)((tot + 127) / 128);
+        if (h->ops->elem_size == 8) k_yref_table_get<double><<<grid, 128, 0, h->stream>>>(h->batch, api_ref(h), stage, dim, d);
+        else k_yref_table_get<float><<<grid, 128, 0, h->stream>>>(h->batch, api_ref(h), stage, dim, d);
+        CK(cudaGetLastError()); h->launches++;
+        return stage_out_end(h, 1, out, (size_t)h->batch * dim, on_device);
+    }
     CK(field_xfer(h, field, stage, d, dim, dim, 0));
     return stage_out_end(h, 1, out, (size_t)h->batch * dim, on_device);
 }
@@ -708,6 +761,7 @@ int bnmpc_set_yref_all(void* handle, const double* value, int on_device) {
     Handle* h = (Handle*)handle;
     if (!h || !value) return fail(BNMPC_E_ARG, "NULL argument");
     if (use_device(h)) return BNMPC_E_CUDA;
+    h->tab_sel = false;            // the uploaded window is the yref source again
     const int N = h->cfg.horizon;
     const size_t per = (size_t)N * (h->ops->nx + h->ops->nu) + h->ops->nx;
     if (h->ops->elem_size == 8) {   // the state keeps yref in exactly this layout: a plain copy, no kernel
@@ -725,6 +779,45 @@ int bnmpc_set_yref_all(void* handle, const double* value, int on_device) {
     return 0;
 }
 
+int bnmpc_set_ref_table(void* handle, const double* table, int rows, int cols, int layout, int on_device) {
+    Handle* h = (Handle*)handle;
+    if (!h) return fail(BNMPC_E_ARG, "NULL handle");
+    if (table) {
+        if (layout != 1 && layout != 2) return fail(BNMPC_E_ARG, "layout must be 1 (one [rows][cols] table shared by all instances) or 2 ([batch][rows][cols], instance-major)");
+        if (cols < h->ops->nx + h->ops->nu) return fail(BNMPC_E_ARG, "cols must be >= nx + nu: a row is [xref | uref | ignored]");
+        if (rows < h->cfg.horizon + 1) return fail(BNMPC_E_ARG, "rows must be >= N + 1: a window is N + 1 rows");
+    }
+    if (use_device(h)) return BNMPC_E_CUDA;
+    // the window the next solve would read stays what it is: if the old table is selected it becomes the stored yref
+    if (int rc = materialise_window(h)) return rc;
+    if (!table) {
+        if (h->tab) { CK(cudaStreamSynchronize(h->stream)); CK(cudaFree(h->tab)); }
+        h->tab = nullptr; h->tab_cap = 0; h->tab_rows = h->tab_cols = 0;
+        return 0;
+    }
+    const size_t count = (size_t)(layout == 1 ? 1 : h->batch) * rows * cols;
+    if (h->tab_cap < count) {
+        CK(cudaStreamSynchronize(h->stream));         // (kernels already enqueued may still read the old table)
+        if (h->tab) CK(cudaFree(h->tab));
+        h->tab = nullptr; h->tab_cap = 0;
+        CK(cudaMalloc(&h->tab, count * sizeof(double)));
+        h->tab_cap = count;
+    }
+    h->tab_rows = rows; h->tab_cols = cols; h->tab_shared = layout == 1;
+    CK(cudaMemcpyAsync(h->tab, table, count * sizeof(double), on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));             // the caller's buffer is free when this returns
+    return 0;
+}
+
+int bnmpc_set_yref_row(void* handle, int row) {
+    Handle* h = (Handle*)handle;
+    if (!h) return fail(BNMPC_E_ARG, "NULL handle");
+    if (!h->tab) return fail(BNMPC_E_ARG, "no reference table bound (bnmpc_set_ref_table)");
+    if (row < 0 || row + h->cfg.horizon >= h->tab_rows) return fail(BNMPC_E_ARG, "row out of range: needs 0 <= row and row + N < rows");
+    h->tab_sel = true; h->tab_row = row;
+    return 0;
+}
+
 int bnmpc_reset(void* handle) {
     Handle* h = (Handle*)handle;
     if (!h) return fail(BNMPC_E_ARG, "NULL handle");
@@ -739,7 +832,7 @@ int bnmpc_solve(void* handle) {
     if (int rc = refresh_order(h)) return rc;
     int* q;
     if (int rc = next_queue(h, &q)) return rc;
-    CK((h->gs.BND ? h->ops->solve_sb : h->ops->solve)(h->gs, h->opts, h->ctas, h->warps, q, h->stream)); h->launches++;
+    CK((h->gs.BND ? h->ops->solve_sb : h->ops->solve)(h->gs, h->opts, api_ref(h), h->ctas, h->warps, q, h->stream)); h->launches++;
     return 0;
 }
 
@@ -761,7 +854,7 @@ int bnmpc_solve_for_x0(void* handle, const double* x0, double* u0, int32_t* stat
     if (int rc = refresh_order(h)) return rc;
     int* q;
     if (int rc = next_queue(h, &q)) return rc;
-    CK((h->gs.BND ? h->ops->solve_sb : h->ops->solve)(h->gs, h->opts, h->ctas, h->warps, q, h->stream)); h->launches++;
+    CK((h->gs.BND ? h->ops->solve_sb : h->ops->solve)(h->gs, h->opts, api_ref(h), h->ctas, h->warps, q, h->stream)); h->launches++;
     if (u0) CK(cudaMemcpyAsync(u0, h->gs.U0, sizeof(double) * B * nu, out, h->stream));   // gathered by the solve kernel
     if (status) CK(cudaMemcpyAsync(status, h->gs.status, sizeof(int32_t) * B, out, h->stream));
     if (!on_device) CK(cudaStreamSynchronize(h->stream));
@@ -799,7 +892,7 @@ int bnmpc_step_for_x0(void* handle, const double* x0, const double* eps, const d
     if (int rc = refresh_order(h)) return rc;
     int* q;
     if (int rc = next_queue(h, &q)) return rc;
-    CK((h->gs.BND ? h->ops->solve_sb : h->ops->solve)(h->gs, h->opts, h->ctas, h->warps, q, h->stream)); h->launches++;
+    CK((h->gs.BND ? h->ops->solve_sb : h->ops->solve)(h->gs, h->opts, api_ref(h), h->ctas, h->warps, q, h->stream)); h->launches++;
     // Converter + plant step + noise on the device, results staged as x_next | u_plant
     double* dout;
     if (int rc = stage_out_begin(h, 1, nullptr, n0 + (size_t)B * 2, 0, &dout)) return rc;

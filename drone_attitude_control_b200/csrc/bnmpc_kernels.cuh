@@ -54,10 +54,11 @@ struct ModelOps {
     int max_wpg, max_warps;                                         // largest warp group per instance the closed-loop kernel was built for; launch bound
     size_t (*smem_bytes)(int N);                                    // dynamic shared memory of one instance (one warp)
     int (*tmem_cols)(int N, int warps, int wpg);                    // tensor-memory columns a CTA of `warps` allocates (0 = too many)
-    cudaError_t (*solve)(const GsAny&, const Opts&, int ctas, int warps, int* queue, cudaStream_t);
+    // `tab`: the handle's bound reference table and window row when it is the yref source (ApiRef::ref == nullptr: Gs::YREF)
+    cudaError_t (*solve)(const GsAny&, const Opts&, const ApiRef& tab, int ctas, int warps, int* queue, cudaStream_t);
     // the same for handles whose instances carry per-stage bounds (GsAny::BND): a second instantiation of the solve kernel, so
     // that the lookup costs the common case nothing
-    cudaError_t (*solve_sb)(const GsAny&, const Opts&, int ctas, int warps, int* queue, cudaStream_t);
+    cudaError_t (*solve_sb)(const GsAny&, const Opts&, const ApiRef& tab, int ctas, int warps, int* queue, cudaStream_t);
     cudaError_t (*loop_step)(const GsAny&, const Opts&, const LoopArgs&, int ctas, int warps, int wpg, int* queue, cudaStream_t);
     // slotted lockstep schedule (bnmpc_lockstep.cuh): LoopArgs::n_steps control steps per launch, tickets of LoopArgs::chunk steps
     cudaError_t (*loop_ls)(const GsAny&, const Opts&, const LoopArgs&, int ctas, int warps, int* queue, cudaStream_t);
@@ -284,12 +285,12 @@ struct DevTickets {
 
 template <class M, class T, bool SB>
 __global__ void __launch_bounds__(32 * LaunchShape<M, T>::MAX_WARPS, 1)
-k_solve(const __grid_constant__ Gs<T> gs, const __grid_constant__ Opts o, int* queue, int tmem_cols) {
+k_solve(const __grid_constant__ Gs<T> gs, const __grid_constant__ Opts o, const __grid_constant__ ApiRef tab, int* queue, int tmem_cols) {
     const uint32_t tbase = tmem_alloc_cta(tmem_cols);
     const WarpGroup<32> g;
     const TmemPriv<M, T, SB> ps{TmemPriv<M, T, SB>::warp_base(tbase, o.N)};
     Solver<M, T, WarpGroup<32>, TmemPriv<M, T, SB>> sv(nullptr, warp_smem_off(o.smem_stride), o, g, ps);
-    for (int inst = next_instance(queue, o.order, gs.B); inst < gs.B; inst = next_instance(queue, o.order, gs.B)) api_solve<M, T>(sv, inst, gs);
+    for (int inst = next_instance(queue, o.order, gs.B); inst < gs.B; inst = next_instance(queue, o.order, gs.B)) api_solve<M, T>(sv, inst, gs, tab);
     tmem_free_cta(tbase, tmem_cols);
 }
 
@@ -481,16 +482,16 @@ struct OpsImpl {
             return e == cudaSuccess ? (long)fa.sharedSizeBytes : -1;
         }
     }
-    static cudaError_t solve(const GsAny& a, const Opts& o_, int ctas, int warps, int* queue, cudaStream_t st) {
+    static cudaError_t solve(const GsAny& a, const Opts& o_, const ApiRef& tab, int ctas, int warps, int* queue, cudaStream_t st) {
         Opts o = o_;
         o.smem_stride = (int)(smem_bytes(o.N) / sizeof(T));
-        k_solve<M, T, false><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, queue, tmem_cols(o.N, warps, 1));
+        k_solve<M, T, false><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, tab, queue, tmem_cols(o.N, warps, 1));
         return cudaGetLastError();
     }
-    static cudaError_t solve_sb(const GsAny& a, const Opts& o_, int ctas, int warps, int* queue, cudaStream_t st) {
+    static cudaError_t solve_sb(const GsAny& a, const Opts& o_, const ApiRef& tab, int ctas, int warps, int* queue, cudaStream_t st) {
         Opts o = o_;
         o.smem_stride = (int)(smem_bytes(o.N) / sizeof(T));
-        k_solve<M, T, true><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, queue, tmem_cols(o.N, warps, 1));
+        k_solve<M, T, true><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, tab, queue, tmem_cols(o.N, warps, 1));
         return cudaGetLastError();
     }
     // `warps` = instances per CTA, each run by a group of wpg warps

@@ -248,14 +248,34 @@ BN_HD void closed_loop_chunk(Solver<M, T, G, PS>& sv, int ticket, const Gs<T>& g
     if (s1 < a.step + a.n_steps) wq.publish(inst, s1);
 }
 
-// one instance, one ocp_solver.solve() with the x0 / yref / p stored through the API
+// The reference table bound to a handle for the solve() path (bnmpc_set_ref_table + bnmpc_set_yref_row): OCP.set_up_ocp(row,
+// xref, uref) with yref_k = table row `row + k`, columns [xref (NX) | uref (NU) | ignored].  ref == nullptr: the yref
+// stored in Gs::YREF.  The table is FP64 in both precisions; Solver::yref_at converts what it reads.
+struct ApiRef {
+    const double* ref;   // [rows][cols] shared by all instances, or [B][rows][cols] (instance-major)
+    int rows, cols;
+    int shared;          // 1 = one table for all instances, 0 = one table per instance
+    int row;             // first row of the window
+};
+
+// row `row + k` of instance inst's table
+BN_HD const double* api_ref_row(const ApiRef& t, int inst, int k) {
+    return t.ref + (t.shared ? (size_t)0 : (size_t)inst * t.rows * t.cols) + (size_t)(t.row + k) * t.cols;
+}
+
+// one instance, one ocp_solver.solve() with the x0 / yref / p stored through the API (yref from `tab` when it has a table)
 template <class M, class T, class G, class PS>
-BN_HD void api_solve(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs) {
+BN_HD void api_solve(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs, const ApiRef& tab = ApiRef{nullptr, 0, 0, 0, 0}) {
     constexpr int NX = M::NX, NU = M::NU, NP = M::NP;
     YrefSrc ys;
     ys.ref = nullptr; ys.ref_rs = 0; ys.ref_cs = 0; ys.ref_off = 0; ys.row0 = 0; ys.circle_n = 0;
-    {
+    if (tab.ref) {
+        ys.yref = nullptr; ys.ref = tab.ref; ys.ref_rs = (size_t)tab.cols; ys.ref_cs = 1; ys.row0 = tab.row;
+        ys.ref_off = tab.shared ? (size_t)0 : (size_t)inst * tab.rows * tab.cols;
+    } else {
         ys.yref = gs.YREF + (size_t)inst * (gs.N * (NU + NX) + NX);
+    }
+    {
         T p[NP];
 #pragma unroll
         for (int j = 0; j < NP; j++) p[j] = gs.PAR[(size_t)inst * NP + j];

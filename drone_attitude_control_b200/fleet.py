@@ -38,7 +38,8 @@ class SolverFleet:
 
     def __init__(self, model='force', batch=1, groups=4, device=0, solver_factory=None, **solver_kw):
         """solver_factory(batch) -> solver object (default: a BatchedAcadosOcpSolver of `model` on a CUDA stream of its own);
-        anything with set_yref_all / step_into / synchronize / reset works (the CPU tests drive the pipeline with a recorder)."""
+        anything with set_yref_all / step_into / synchronize / reset works, plus set_ref_table / set_yref_row for step_at (the CPU
+        tests drive the pipeline with a recorder)."""
         self.bounds = group_bounds(batch, groups)
         self.groups = len(self.bounds) - 1
         self.batch = int(batch)
@@ -74,6 +75,24 @@ class SolverFleet:
         outputs are valid after `wait(g)` / `synchronize()` - or inside `on_results(g, lo, hi)`, which the next call of `step`
         invokes for each sub-fleet once its previous step is back on the host and before its next one is enqueued (the place
         of the reference's status check and logging, src/force_model/controller.py:33-41)."""
+        self._step(lambda s, lo, hi: s.set_yref_all(yref[lo:hi]), x0, eps, u0, u_plant, status, x_next, p_plant, on_results)
+
+    def set_ref_table(self, table):
+        """Bind the reference trajectory to every sub-fleet once (BatchedAcadosOcpSolver.set_ref_table): a shared table
+        [rows, cols] goes to all of them, a per-drone table [B, rows, cols] gives sub-fleet g its rows lo_g:hi_g."""
+        per_drone = table.ndim == 3
+        if per_drone and table.shape[0] != self.batch:
+            raise ValueError(f'per-drone table: expected {self.batch} tables, got {table.shape[0]}')
+        for g, s in enumerate(self.solvers):
+            lo, hi = self.bounds[g], self.bounds[g + 1]
+            s.set_ref_table(table[lo:hi] if per_drone else table)
+
+    def step_at(self, i, x0, eps, u0, u_plant, status, x_next, p_plant=None, on_results=None):
+        """`step` with the reference window taken from the table of set_ref_table at row i (OCP.set_up_ocp(i, xref, uref),
+        bnmpc_set_yref_row + bnmpc_step_for_x0 per sub-fleet): no reference upload.  Same buffers, pipeline and hook."""
+        self._step(lambda s, lo, hi: s.set_yref_row(i), x0, eps, u0, u_plant, status, x_next, p_plant, on_results)
+
+    def _step(self, set_ref, x0, eps, u0, u_plant, status, x_next, p_plant, on_results):
         for g, s in enumerate(self.solvers):
             lo, hi = self.bounds[g], self.bounds[g + 1]
             if self._pending[g]:
@@ -81,7 +100,7 @@ class SolverFleet:
                 self._pending[g] = False
                 if on_results is not None:
                     on_results(g, lo, hi)
-            s.set_yref_all(yref[lo:hi])
+            set_ref(s, lo, hi)
             s.step_into(x0[lo:hi], None if eps is None else eps[lo:hi], u0[lo:hi], u_plant[lo:hi], status[lo:hi], x_next[lo:hi],
                         p_plant_host=None if p_plant is None else p_plant[lo:hi], wait=False)
             self._pending[g] = True

@@ -133,8 +133,30 @@ int64_t bnmpc_workspace_bytes(void* handle);
 int bnmpc_set(void* handle, int stage, int field, const double* value, int on_device);
 /* ocp_solver.get(stage, field); out is AoS [batch][dim]. */
 int bnmpc_get(void* handle, int stage, int field, double* out, int on_device);
-/* OCP.set_up_ocp in one call (src/force_model/ocp.py:117-122): AoS [batch][N*ny + ny_e] = yref_0 .. yref_{N-1}, yref_N */
+/* OCP.set_up_ocp in one call (src/force_model/ocp.py:117-122): AoS [batch][N*ny + ny_e] = yref_0 .. yref_{N-1}, yref_N.
+ * Makes this stored yref the source of the solves again (after bnmpc_set_yref_row). */
 int bnmpc_set_yref_all(void* handle, const double* value, int on_device);
+/* The reference as the reference hands it to OCP.set_up_ocp (src/force_model/ocp.py:117-122): the whole trajectory, bound
+ * once, plus a row index per control step (bnmpc_set_yref_row) instead of a window upload per step.
+ *
+ * bnmpc_set_ref_table copies `table` into memory the handle owns (cudaMemcpyAsync on the handle's stream; the call returns
+ * when the copy is done, no pointer is retained) and counts it in bnmpc_workspace_bytes.  layout 1 = one [rows][cols] table
+ * shared by all instances, 2 = [batch][rows][cols] (instance-major) - the numbering of bnmpc_closed_loop_args.ref_shared.
+ * Row r = [xref_r (nx) | uref_r (nu) | ignored], cols >= nx + nu (the 8-column gen_circle_traj table of force / jerk, the
+ * 14-column helix table of the 3-D model), rows >= N + 1.  The table stays FP64 in FP32 mode: the solve rounds what it
+ * reads exactly as bnmpc_set_yref_all rounds the uploaded window, so both ways give bit-identical results.
+ * table == NULL releases the binding.  Binding does not change the yref source; binding a new table or releasing it while
+ * the old one is selected first stores the current window as the yref (one gather kernel), so the next solve sees the
+ * same yref either way.  BNMPC_E_ARG for a layout other than 1 or 2, cols < nx + nu or rows < N + 1. */
+int bnmpc_set_ref_table(void* handle, const double* table, int rows, int cols, int layout, int on_device);
+/* OCP.set_up_ocp(row, xref, uref) for all instances: yref_k = [xref[row+k], uref[row+k]] (k < N), yref_N = xref[row+N],
+ * read by bnmpc_solve / bnmpc_solve_for_x0 / bnmpc_step_for_x0 straight from the bound table - no copy, no kernel - until
+ * bnmpc_set_yref_all or bnmpc_set(k, 'yref', v) is called.  bnmpc_set(k, 'yref', v) while the table is selected first
+ * stores the current window as the yref (one gather kernel), then writes stage k: the same as bnmpc_set_yref_all(window)
+ * followed by that set.  bnmpc_get(k, 'yref') while the table is selected returns the window's stage k (the values the
+ * solve reads: rounded to float in FP32) and changes no handle state.  BNMPC_E_ARG with no table bound, or unless
+ * 0 <= row and row + N < rows. */
+int bnmpc_set_yref_row(void* handle, int row);
 /* zero the primal iterate and multipliers (state of a freshly created acados solver) */
 int bnmpc_reset(void* handle);
 /* ocp_solver.solve() (src/force_model/controller.py:32): one acados-style SQP run per instance from the stored
