@@ -74,6 +74,8 @@ def lib():
         'bnmpc_solve_for_x0': (C.c_int, [vp, dp, dp, vp, C.c_int]),
         'bnmpc_sim_step': (C.c_int, [vp, C.c_int, dp, dp, dp, dp, dp, C.c_int]),
         'bnmpc_step_for_x0': (C.c_int, [vp, dp, dp, dp, dp, dp, vp, dp, C.c_int]),
+        'bnmpc_eval_sens_x0': (C.c_int, [vp, C.c_int, dp, dp, C.c_int]),
+        'bnmpc_eval_adjoint_sens': (C.c_int, [vp, dp, dp, dp, dp, C.c_int]),
         'bnmpc_closed_loop_init': (C.c_int, [vp, dp, dp, dp]),
         'bnmpc_closed_loop_run': (C.c_int, [vp, C.POINTER(ClosedLoopArgs)]),
         'bnmpc_closed_loop_state': (C.c_int, [vp, dp, dp, dp, dp]),

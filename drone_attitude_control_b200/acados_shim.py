@@ -6,6 +6,7 @@ The reference drives acados through `acados_template.AcadosOcpSolver` / `AcadosS
 
     set(stage, field, value)   get(stage, field)   solve() -> status   get_stats(name)   print_statistics()
     solve_for_x0(x0_bar)       get_cost()          reset()
+    eval_solution_sensitivity()             eval_adjoint_solution_sensitivity(seed_x, seed_u)
 
 `value` is a `[batch, dim]` tensor (CUDA or CPU) or numpy array; with batch == 1 a plain `(dim,)` numpy vector is
 accepted and `get` returns one, so the reference's `follow_trajectory` runs against this class unchanged apart from the
@@ -52,6 +53,7 @@ class BatchedAcadosOcpSolver:
         self.nx, self.nu, self.ny, self.ny_e, self.N, self.np_, self.nblk = [int(v) for v in dims]
         self._bind_stream()
         self._time_tot = 0.0
+        self.solve_count = 0        # solves (and resets) so far: a sensitivity belongs to the solution of one of them
 
     # -- plumbing ------------------------------------------------------------------------------------------------------
     def _bind_stream(self):
@@ -166,6 +168,7 @@ class BatchedAcadosOcpSolver:
         ev0 = torch.cuda.Event(enable_timing=True); ev1 = torch.cuda.Event(enable_timing=True)
         ev0.record(self._stream)
         check(lib().bnmpc_solve(self._h))
+        self.solve_count += 1
         ev1.record(self._stream)
         self._ev = (ev0, ev1)
         st = self.get_stats('status')
@@ -211,6 +214,7 @@ class BatchedAcadosOcpSolver:
         ev0 = torch.cuda.Event(enable_timing=True); ev1 = torch.cuda.Event(enable_timing=True)
         ev0.record(self._stream)
         check(lib().bnmpc_solve_for_x0(self._h, ptr, up, sp, on_dev))
+        self.solve_count += 1
         ev1.record(self._stream)
         self._ev = (ev0, ev1)
         self._keep = keep
@@ -229,11 +233,13 @@ class BatchedAcadosOcpSolver:
         of the next step's reference window on another stream) then runs behind this step's x0 upload, not in front."""
         check(lib().bnmpc_solve_for_x0(self._h, C.c_void_p(x0_host.data_ptr()), C.c_void_p(u0_host.data_ptr()),
                                        C.c_void_p(status_host.data_ptr()), 0 if wait else 2))
+        self.solve_count += 1
 
     def solve_for_x0_device(self, x0_dev, u0_dev, status_dev):
         """Same with device tensors: everything stays on the solver's stream, nothing synchronises."""
         check(lib().bnmpc_solve_for_x0(self._h, C.c_void_p(x0_dev.data_ptr()), C.c_void_p(u0_dev.data_ptr()),
                                        C.c_void_p(status_dev.data_ptr()), 1))
+        self.solve_count += 1
 
     def step_into(self, x0_host, eps_host, u0_host, up_host, status_host, xn_host, p_plant_host=None, wait=True):
         """One iteration of the reference's follow_trajectory for all drones in one call (bnmpc_step_for_x0): x0 embedding,
@@ -242,12 +248,14 @@ class BatchedAcadosOcpSolver:
         ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
         check(lib().bnmpc_step_for_x0(self._h, ptr(x0_host), ptr(eps_host), ptr(p_plant_host), ptr(u0_host), ptr(up_host),
                                       ptr(status_host), ptr(xn_host), 0 if wait else 2))
+        self.solve_count += 1
 
     def step_device(self, x0_dev, eps_dev, u0_dev, up_dev, status_dev, xn_dev, p_plant_dev=None):
         """step_into with device tensors: everything is enqueued on the solver's stream, nothing synchronises."""
         ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
         check(lib().bnmpc_step_for_x0(self._h, ptr(x0_dev), ptr(eps_dev), ptr(p_plant_dev), ptr(u0_dev), ptr(up_dev),
                                       ptr(status_dev), ptr(xn_dev), 1))
+        self.solve_count += 1
 
     def simulate_next_x_into(self, x_host, u_host, eps_host, xn_host, p_plant_host=None, wait=True):
         """OCP.simulate_next_x (src/force_model/ocp.py:106-115, src/jerk_model/ocp.py:106-116) for all drones with the plant
@@ -274,8 +282,64 @@ class BatchedAcadosOcpSolver:
             self.numpy_io = io
         return float(tot[0]) if self.batch == 1 else tot
 
+    # -- solution sensitivities (acados' eval_solution_sensitivity; models force, jerk and force_dense) --------------------
+    def eval_solution_sensitivity(self, stages=None, with_respect_to='initial_state'):
+        """d x_k / d x0 and d u_k / d x0 at the solution of the last solve (bnmpc_eval_sens_x0), stages 0 .. stages-1
+        (default N + 1): returns (sens_x [batch, stages, nx, nx], sens_u [batch, min(stages, N), nu, nx]) - torch tensors on
+        the solver's device, or numpy without the batch dimension when batch == 1, as get() does.  sens_u[:, 0] is the
+        feedback gain of u0.  Rows of an instance whose last solve did not succeed are NaN.  Only 'initial_state' is
+        supported (sensitivities with respect to the parameters p are not)."""
+        if with_respect_to != 'initial_state':
+            raise ValueError(f"with_respect_to={with_respect_to!r}: only 'initial_state' is supported")
+        stages = self.N + 1 if stages is None else int(stages)
+        if not 1 <= stages <= self.N + 1:
+            raise ValueError(f'stages must be within 1 .. {self.N + 1}, got {stages}')
+        shapes = ((self.batch, stages, self.nx, self.nx), (self.batch, min(stages, self.N), self.nu, self.nx))
+        if self.numpy_io:
+            sx, su = np.empty(shapes[0]), np.empty(shapes[1])
+            check(lib().bnmpc_eval_sens_x0(self._h, stages, C.c_void_p(sx.ctypes.data), C.c_void_p(su.ctypes.data), 0))
+            return (sx[0], su[0]) if self.batch == 1 else (sx, su)
+        sx, su = (torch.empty(sh, dtype=torch.float64, device=self.device) for sh in shapes)
+        check(lib().bnmpc_eval_sens_x0(self._h, stages, C.c_void_p(sx.data_ptr()), C.c_void_p(su.data_ptr()), 1))
+        return sx, su
+
+    def _seed(self, v, shape):
+        if v is None:
+            return None
+        t = v.detach().to(torch.float64) if isinstance(v, torch.Tensor) else torch.from_numpy(np.asarray(v, dtype=np.float64))
+        if t.dim() == len(shape) - 1 and self.batch == 1:
+            t = t[None]
+        if tuple(t.shape) != shape:
+            raise ValueError(f'expected seed shape {shape}, got {tuple(v.shape)}')
+        return t.to(self.device).contiguous()
+
+    def adjoint_device(self, seed_x=None, seed_u=None):
+        """eval_adjoint_solution_sensitivity with device tensors in and out, asynchronous on the solver's stream."""
+        sx = self._seed(seed_x, (self.batch, self.N + 1, self.nx))
+        su = self._seed(seed_u, (self.batch, self.N, self.nu))
+        if sx is None and su is None:
+            raise ValueError('seed_x and seed_u are both None')
+        gx = torch.empty((self.batch, self.nx), dtype=torch.float64, device=self.device)
+        gy = torch.empty((self.batch, self.N * self.ny + self.ny_e), dtype=torch.float64, device=self.device)
+        ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        check(lib().bnmpc_eval_adjoint_sens(self._h, ptr(sx), ptr(su), ptr(gx), ptr(gy), 1))
+        self._keep = (sx, su)
+        return gx, gy
+
+    def eval_adjoint_solution_sensitivity(self, seed_x=None, seed_u=None):
+        """Adjoint of eval_solution_sensitivity (bnmpc_eval_adjoint_sens): seed_x [batch, N+1, nx], seed_u [batch, N, nu]
+        (None = 0, not both) -> (grad_x0 [batch, nx], grad_yref [batch, N*ny + ny_e]) = sum over the stages of the
+        sensitivities' transposes times the seeds, with respect to x0 and to the set_yref_all window.  One linear solve per
+        drone whatever the seed.  Output types as for eval_solution_sensitivity."""
+        gx, gy = self.adjoint_device(seed_x, seed_u)
+        if self.numpy_io:
+            gx, gy = gx.cpu().numpy(), gy.cpu().numpy()
+            return (gx[0], gy[0]) if self.batch == 1 else (gx, gy)
+        return gx, gy
+
     def reset(self):
         check(lib().bnmpc_reset(self._h))
+        self.solve_count += 1
 
     def synchronize(self):
         check(lib().bnmpc_synchronize(self._h))

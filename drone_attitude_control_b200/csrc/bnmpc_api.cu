@@ -54,6 +54,7 @@ struct Handle {
     double* tab; size_t tab_cap;   // device copy, its capacity in doubles
     int tab_rows, tab_cols, tab_shared;
     bool tab_sel; int tab_row;     // the table (window at tab_row) is the yref source of the solves, not Gs::YREF
+    double* sens_stage; size_t sens_cap;   // device staging of the sensitivity evaluations with host buffers, its capacity in doubles
 };
 
 const ModelOps* pick_ops(int model, int precision) {
@@ -475,6 +476,26 @@ int materialise_window(Handle* h) {
     return 0;
 }
 
+// staging area of a sensitivity evaluation with host buffers: `count` doubles, handle-owned, grown on demand
+int sens_staging(Handle* h, size_t count, double** out) {
+    if (h->sens_cap < count) {
+        CK(cudaStreamSynchronize(h->stream));
+        if (h->sens_stage) CK(cudaFree(h->sens_stage));
+        h->sens_stage = nullptr; h->sens_cap = 0;
+        CK(cudaMalloc(&h->sens_stage, count * sizeof(double)));
+        h->sens_cap = count;
+    }
+    *out = h->sens_stage;
+    return 0;
+}
+
+int launch_sens(Handle* h, const SensArgs& a, int mode) {
+    int* q;
+    if (int rc = next_queue(h, &q)) return rc;
+    CK(h->ops->sens(h->gs, h->opts, a, mode, h->ctas, h->warps, q, h->stream)); h->launches++;
+    return 0;
+}
+
 int reset_iterate(Handle* h) {
     const size_t es = h->ops->elem_size, B = h->batch;
     CK(cudaMemsetAsync(h->gs.V, 0, B * h->nV * es, h->stream));
@@ -674,6 +695,7 @@ int bnmpc_destroy(void* handle) {
     if (h->gs.U0) cudaFree(h->gs.U0);
     if (h->gs.BND) cudaFree(h->gs.BND);
     if (h->tab) cudaFree(h->tab);
+    if (h->sens_stage) cudaFree(h->sens_stage);
     for (int i = 0; i < 4; i++) if (h->stage[i]) cudaFree(h->stage[i]);
     if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -708,7 +730,8 @@ int bnmpc_dims(void* handle, int32_t dims[7]) {
 
 int64_t bnmpc_workspace_bytes(void* handle) {
     Handle* h = (Handle*)handle;
-    return h ? (int64_t)(h->gs_bytes + sizeof(int32_t) * 4 * h->batch + sizeof(double) * 11 * h->Bp + sizeof(double) * h->tab_cap) : 0;
+    return h ? (int64_t)(h->gs_bytes + sizeof(int32_t) * 4 * h->batch + sizeof(double) * 11 * h->Bp + sizeof(double) * h->tab_cap +
+                         sizeof(double) * h->sens_cap) : 0;
 }
 
 int bnmpc_set(void* handle, int stage, int field, const double* value, int on_device) {
@@ -858,6 +881,57 @@ int bnmpc_solve_for_x0(void* handle, const double* x0, double* u0, int32_t* stat
     if (u0) CK(cudaMemcpyAsync(u0, h->gs.U0, sizeof(double) * B * nu, out, h->stream));   // gathered by the solve kernel
     if (status) CK(cudaMemcpyAsync(status, h->gs.status, sizeof(int32_t) * B, out, h->stream));
     if (!on_device) CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+int bnmpc_eval_sens_x0(void* handle, int stages, double* sens_x, double* sens_u, int on_device) {
+    Handle* h = (Handle*)handle;
+    if (!h) return fail(BNMPC_E_ARG, "NULL handle");
+    if (!h->ops->sens) return fail(BNMPC_E_UNSUPPORTED, "solution sensitivities need the exact Hessian of the Lagrangian: models FORCE, JERK and FORCE_DENSE only");
+    const int N = h->cfg.horizon;
+    if (stages < 1 || stages > N + 1) return fail(BNMPC_E_ARG, "stages must be within 1 .. N+1");
+    if (on_device != 0 && on_device != 1) return fail(BNMPC_E_ARG, "on_device must be 0 or 1");
+    if (use_device(h)) return BNMPC_E_CUDA;
+    const size_t B = h->batch, nx = h->ops->nx, nu = h->ops->nu;
+    const size_t nsx = sens_x ? B * stages * nx * nx : 0, nsu = sens_u ? B * (stages < N ? stages : N) * nu * nx : 0;
+    SensArgs a{stages, sens_x, sens_u, nullptr, nullptr, nullptr, nullptr};
+    double* d = nullptr;
+    if (!on_device) {
+        if (int rc = sens_staging(h, nsx + nsu, &d)) return rc;
+        a.sens_x = sens_x ? d : nullptr; a.sens_u = sens_u ? d + nsx : nullptr;
+    }
+    if (int rc = launch_sens(h, a, 0)) return rc;
+    if (on_device) return 0;
+    if (sens_x) CK(cudaMemcpyAsync(sens_x, d, nsx * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (sens_u) CK(cudaMemcpyAsync(sens_u, d + nsx, nsu * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+int bnmpc_eval_adjoint_sens(void* handle, const double* seed_x, const double* seed_u, double* grad_x0, double* grad_yref, int on_device) {
+    Handle* h = (Handle*)handle;
+    if (!h) return fail(BNMPC_E_ARG, "NULL handle");
+    if (!h->ops->sens) return fail(BNMPC_E_UNSUPPORTED, "solution sensitivities need the exact Hessian of the Lagrangian: models FORCE, JERK and FORCE_DENSE only");
+    if (!seed_x && !seed_u) return fail(BNMPC_E_ARG, "seed_x and seed_u are both NULL");
+    if (on_device != 0 && on_device != 1) return fail(BNMPC_E_ARG, "on_device must be 0 or 1");
+    if (use_device(h)) return BNMPC_E_CUDA;
+    const size_t B = h->batch, nx = h->ops->nx, nu = h->ops->nu, N = h->cfg.horizon;
+    const size_t nsx = seed_x ? B * (N + 1) * nx : 0, nsu = seed_u ? B * N * nu : 0;
+    const size_t ngx = grad_x0 ? B * nx : 0, ngy = grad_yref ? B * (N * (nx + nu) + nx) : 0;
+    SensArgs a{0, nullptr, nullptr, seed_x, seed_u, grad_x0, grad_yref};
+    double* d = nullptr;
+    if (!on_device) {       // one staging area: seed_x | seed_u | grad_x0 | grad_yref
+        if (int rc = sens_staging(h, nsx + nsu + ngx + ngy, &d)) return rc;
+        if (seed_x) CK(cudaMemcpyAsync(d, seed_x, nsx * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        if (seed_u) CK(cudaMemcpyAsync(d + nsx, seed_u, nsu * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        a.seed_x = seed_x ? d : nullptr; a.seed_u = seed_u ? d + nsx : nullptr;
+        a.grad_x0 = grad_x0 ? d + nsx + nsu : nullptr; a.grad_yref = grad_yref ? d + nsx + nsu + ngx : nullptr;
+    }
+    if (int rc = launch_sens(h, a, 1)) return rc;
+    if (on_device) return 0;
+    if (grad_x0) CK(cudaMemcpyAsync(grad_x0, a.grad_x0, ngx * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (grad_yref) CK(cudaMemcpyAsync(grad_yref, a.grad_yref, ngy * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
 

@@ -65,6 +65,9 @@ struct ModelOps {
     // warps per CTA and warps per instance (wpg; instances in flight per SM = warps / wpg), warps = 0: does not fit
     cudaError_t (*cta_shape)(int N, int* warps, int* wpg);
     long (*loop_static_bytes)(int wpg);                             // static shared memory of the closed-loop kernel (-1: none)
+    // solution sensitivities at the stored solutions, mode 0: d(x_k, u_k) / d x0, 1: adjoint (bnmpc_eval_sens_x0 /
+    // bnmpc_eval_adjoint_sens); nullptr for the models whose Gauss-Newton Hessian is not the Lagrangian's (THRUST, ATT)
+    cudaError_t (*sens)(const GsAny&, const Opts&, const SensArgs&, int mode, int ctas, int warps, int* queue, cudaStream_t);
 };
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -294,6 +297,21 @@ k_solve(const __grid_constant__ Gs<T> gs, const __grid_constant__ Opts o, const 
     tmem_free_cta(tbase, tmem_cols);
 }
 
+// Solution sensitivities at the stored solutions, MODE 0: forward in x0 (api_sens_x0), 1: adjoint (api_sens_adj).  The
+// launch shape, work queue and shared-memory layout of k_solve, with the per-stage-bound lookup compiled in.  The passes
+// involved (factorisation, Newton solve) keep nothing in the lane-private record, so the kernel allocates no tensor memory.
+template <class M, class T, int MODE>
+__global__ void __launch_bounds__(32 * LaunchShape<M, T>::MAX_WARPS, 1)
+k_sens(const __grid_constant__ Gs<T> gs, const __grid_constant__ Opts o, const __grid_constant__ SensArgs a, int* queue) {
+    const WarpGroup<32> g;
+    const TmemPriv<M, T, true> ps{0u};
+    Solver<M, T, WarpGroup<32>, TmemPriv<M, T, true>> sv(nullptr, warp_smem_off(o.smem_stride), o, g, ps);
+    for (int inst = next_instance(queue, nullptr, gs.B); inst < gs.B; inst = next_instance(queue, nullptr, gs.B)) {
+        if constexpr (MODE == 0) api_sens_x0<M, T>(sv, inst, gs, a);
+        else api_sens_adj<M, T>(sv, inst, gs, a);
+    }
+}
+
 // WPG warps per instance (see WarpGroup): 1 at the reference horizon, 2 / 4 where the horizon leaves room for only 8 / 4
 // instances per SM
 template <class M, class T, int WPG>
@@ -454,6 +472,12 @@ struct OpsImpl {
         if (e != cudaSuccess) return e;
         e = prep(k_solve<M, T, true>, 0);
         if (e != cudaSuccess) return e;
+        if constexpr (M::JAC_CONST) {
+            e = prep(k_sens<M, T, 0>, 0);
+            if (e != cudaSuccess) return e;
+            e = prep(k_sens<M, T, 1>, 0);
+            if (e != cudaSuccess) return e;
+        }
         int dev = 0, optin = 0;
         e = cudaGetDevice(&dev);
         if (e != cudaSuccess) return e;
@@ -519,9 +543,20 @@ struct OpsImpl {
         return cudaGetLastError();
         }
     }
+    static cudaError_t sens(const GsAny& a, const Opts& o_, const SensArgs& sa, int mode, int ctas, int warps, int* queue, cudaStream_t st) {
+        if constexpr (!M::JAC_CONST) return cudaErrorNotSupported;
+        else {
+        Opts o = o_;
+        o.smem_stride = (int)(smem_bytes(o.N) / sizeof(T));
+        if (mode == 0) k_sens<M, T, 0><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, sa, queue);
+        else k_sens<M, T, 1><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, sa, queue);
+        return cudaGetLastError();
+        }
+    }
     static ModelOps make(int kind) {
         return ModelOps{M::name(), M::NX, M::NU, M::NP, M::NBLK, M::NXB, M::NUB, kind, M::JAC_CONST ? 1 : 0, (int)sizeof(T),
-                        SmLayout<M, false, TmemPriv<M, T>::QB_PRIV>::ROWS, GROUPS ? 4 : 1, LaunchShape<M, T>::MAX_WARPS, &smem_bytes, &tmem_cols, &solve, &solve_sb, &loop_step, &loop_ls, &cta_shape, &loop_static_bytes};
+                        SmLayout<M, false, TmemPriv<M, T>::QB_PRIV>::ROWS, GROUPS ? 4 : 1, LaunchShape<M, T>::MAX_WARPS, &smem_bytes, &tmem_cols, &solve, &solve_sb, &loop_step, &loop_ls, &cta_shape, &loop_static_bytes,
+                        M::JAC_CONST ? &sens : nullptr};
     }
 };
 

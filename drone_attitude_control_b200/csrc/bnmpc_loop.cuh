@@ -293,4 +293,158 @@ BN_HD void api_solve(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs, const A
     sv.g.sync();
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// solution sensitivities at the stored solutions (bnmpc_eval_sens_x0 / bnmpc_eval_adjoint_sens), FP64 in and out
+// ---------------------------------------------------------------------------------------------------------------------
+struct SensArgs {
+    int stages;                     // forward: stages 0 .. stages-1 of sens_x, 0 .. min(stages, N)-1 of sens_u
+    double *sens_x, *sens_u;        // [B][stages][NX][NX] = d x_k / d x0, [B][min(stages, N)][NU][NX] = d u_k / d x0, or NULL
+    const double *seed_x, *seed_u;  // adjoint: [B][N+1][NX], [B][N][NU], NULL = 0
+    double *grad_x0, *grad_yref;    // [B][NX], [B][N*(NX+NU) + NX] (the bnmpc_set_yref_all layout), or NULL
+};
+
+// Binds the instance and factorises its KKT matrix (Solver::sens_factor).  false: the last solve did not succeed or left no
+// multipliers - there is no solution to differentiate and the caller writes NaN rows.
+template <class M, class T, class G, class PS>
+BN_HD bool sens_begin(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs) {
+    constexpr int NX = M::NX, NU = M::NU, NP = M::NP;
+    if (gs.status[inst] != ST_SUCCESS || gs.have_mult[inst] == 0) return false;
+    T p[NP];
+#pragma unroll
+    for (int j = 0; j < NP; j++) p[j] = gs.PAR[(size_t)inst * NP + j];
+    sv.set_par(p);
+    sv.bnd = gs.BND ? gs.BND + (size_t)inst * gs.N * 2 * (NU + NX) : nullptr;
+    sv.sens_factor(gs, inst);
+    return true;
+}
+
+template <class G>
+BN_HD void nan_fill(const G& g, double* p, size_t count) {
+    if (!p) return;
+    for (size_t e = (size_t)g.lane; e < count; e += G::L) p[e] = (double)NAN;
+}
+
+// Forward: x0 enters the QP only through b_0 = A_0 (x0 - x_0) (Solver::build_qp), so direction e_j is one Newton solve with
+// RB = A_0 e_j at stage 0 and a zero gradient; its step is column j of d(x_k, u_k) / d x0.  sens_x[0] = I.
+template <class M, class T, class G, class PS>
+BN_HD void api_sens_x0(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs, const SensArgs& a) {
+    using SL = typename Solver<M, T, G, PS>::SL;
+    constexpr int n = M::NXB, m = M::NUB, s = n + m, NBLK = M::NBLK, NX = M::NX, NU = M::NU;
+    const int N = sv.N, ns = a.stages, nsu = a.stages < N ? a.stages : N;
+    double* sx = a.sens_x ? a.sens_x + (size_t)inst * ns * NX * NX : nullptr;
+    double* su = a.sens_u ? a.sens_u + (size_t)inst * nsu * NU * NX : nullptr;
+    if (!sens_begin(sv, inst, gs)) {
+        nan_fill(sv.g, sx, (size_t)ns * NX * NX);
+        nan_fill(sv.g, su, (size_t)nsu * NU * NX);
+        sv.g.sync();
+        return;
+    }
+    for (int j = 0; j < NX; j++) {
+        const int bj = xblk<M>(j), lj = xloc<M>(j);
+        for (int sb = sv.g.lane; sb < sv.NSB; sb += G::L) {
+            const int k = sb / NBLK, b = sb % NBLK;
+            sv.use_block(b);
+#pragma unroll
+            for (int v = 0; v < s; v++) sv.S(SL::GV + v, sb) = T(0);
+            if (k < N) {
+#pragma unroll
+                for (int r = 0; r < n; r++) {
+                    T e = T(0);      // A_0[r][lj], selected with constant indices so that A stays in registers
+#pragma unroll
+                    for (int c = 0; c < n; c++) if (k == 0 && b == bj && c == lj) e = sv.maA(T(0), T(1), r, c);
+                    sv.S(SL::RB + r, sb) = e;
+                }
+            }
+        }
+        sv.g.sync();
+        sv.sens_solve(ns > 2);
+        for (int sb = sv.g.lane; sb < sv.NSB; sb += G::L) {
+            const int k = sb / NBLK, b = sb % NBLK;
+            if (sx && k < ns) {
+#pragma unroll
+                for (int r = 0; r < n; r++)
+                    sx[((size_t)k * NX + M::xg(b, r)) * NX + j] = k == 0 ? (M::xg(b, r) == j ? 1.0 : 0.0) : double(sv.S(SL::DZA + m + r, sb));
+            }
+            if (su && k < nsu) {
+#pragma unroll
+                for (int c = 0; c < m; c++) su[((size_t)k * NU + M::ug(b, c)) * NX + j] = double(sv.S(SL::DZA + c, sb));
+            }
+        }
+        sv.g.sync();
+    }
+}
+
+// Adjoint: the KKT matrix is symmetric, so the Newton solve with the seed as gradient (RB = 0) gives the vector-Jacobian
+// products.  With that step (dz, dpi): grad_x0 = seed_x[0] + A_0' dpi_0, and since the cost gradient depends on yref through
+// -dt W (stages < N) / -W_e (stage N), grad_yref = -dt W dz / -W_e dz (0 for the x-part of stage 0: x_0 is not a variable).
+template <class M, class T, class G, class PS>
+BN_HD void api_sens_adj(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs, const SensArgs& a) {
+    using SL = typename Solver<M, T, G, PS>::SL;
+    constexpr int n = M::NXB, m = M::NUB, s = n + m, NBLK = M::NBLK, NX = M::NX, NU = M::NU, ny = NX + NU;
+    const int N = sv.N;
+    const double* sdx = a.seed_x ? a.seed_x + (size_t)inst * (N + 1) * NX : nullptr;
+    const double* sdu = a.seed_u ? a.seed_u + (size_t)inst * N * NU : nullptr;
+    double* gx = a.grad_x0 ? a.grad_x0 + (size_t)inst * NX : nullptr;
+    double* gy = a.grad_yref ? a.grad_yref + (size_t)inst * (N * ny + NX) : nullptr;
+    if (!sens_begin(sv, inst, gs)) {
+        nan_fill(sv.g, gx, NX);
+        nan_fill(sv.g, gy, (size_t)N * ny + NX);
+        sv.g.sync();
+        return;
+    }
+    for (int sb = sv.g.lane; sb < sv.NSB; sb += G::L) {
+        const int k = sb / NBLK, b = sb % NBLK;
+#pragma unroll
+        for (int v = 0; v < s; v++) {
+            T sd = T(0);
+            if (sv.has(k, v)) {
+                if (v < m) { if (sdu) sd = T(sdu[(size_t)k * NU + M::ug(b, v)]); }
+                else if (sdx) sd = T(sdx[(size_t)k * NX + M::xg(b, v - m)]);
+            }
+            sv.S(SL::GV + v, sb) = sd;
+        }
+        if (k < N) {
+#pragma unroll
+            for (int r = 0; r < n; r++) sv.S(SL::RB + r, sb) = T(0);
+        }
+    }
+    sv.g.sync();
+    sv.sens_solve(gy != nullptr);
+    if (gx) {
+        for (int b = sv.g.lane; b < NBLK; b += G::L) {
+            sv.use_block(b);
+            const int sb1 = NBLK + b;
+            T dpi[n];       // dpi_0 = p_1 + P_1 dx_1 (the multiplier step of Solver::qp_update)
+#pragma unroll
+            for (int r = 0; r < n; r++) {
+                T d = sv.S(SL::GV + m + r, sb1);
+#pragma unroll
+                for (int l = 0; l < n; l++) d += sv.S(SL::P + sv.pidx(r, l), sb1) * sv.S(SL::DZA + m + l, sb1);
+                dpi[r] = d;
+            }
+#pragma unroll
+            for (int c = 0; c < n; c++) {
+                T acc = sdx ? T(sdx[M::xg(b, c)]) : T(0);
+#pragma unroll
+                for (int r = 0; r < n; r++) acc = sv.maA(acc, dpi[r], r, c);
+                gx[M::xg(b, c)] = double(acc);
+            }
+        }
+    }
+    if (gy) {
+        for (int sb = sv.g.lane; sb < sv.NSB; sb += G::L) {
+            const int k = sb / NBLK, b = sb % NBLK;
+            sv.use_block(b);
+#pragma unroll
+            for (int v = 0; v < s; v++) {
+                if (v < m && k == N) continue;
+                const size_t e = (size_t)k * ny + (v < m ? NX + M::ug(b, v) : M::xg(b, v - m));
+                const T h = k < N ? sv.Hd[v] : sv.He[v - m];
+                gy[e] = sv.has(k, v) ? double(-h * sv.S(SL::DZA + v, sb)) : 0.0;
+            }
+        }
+    }
+    sv.g.sync();
+}
+
 }  // namespace bnmpc

@@ -181,6 +181,25 @@ int bnmpc_solve_for_x0(void* handle, const double* x0, double* u0, int32_t* stat
  * bnmpc_solve_for_x0. */
 int bnmpc_step_for_x0(void* handle, const double* x0, const double* eps, const double* p_plant, double* u0, double* u_plant,
                       int32_t* status, double* x_next, int on_device);
+/* Parametric solution sensitivities at the stored solution of every instance (acados' eval_solution_sensitivity), for the
+ * models whose Gauss-Newton Hessian is the exact Hessian of the Lagrangian (FORCE, JERK, FORCE_DENSE: affine dynamics,
+ * LINEAR_LS cost); BNMPC_E_UNSUPPORTED for THRUST and ATT.  The KKT matrix is the x0-eliminated one of the converged QP with
+ * Hessian diagonal dt W (W_e at stage N) + lam_lb / t_lb + lam_ub / t_ub: the stored multipliers, slacks recomputed from the
+ * stored iterate as t_lb = max(v - lb, t_min), t_ub = max(ub - v, t_min), the instance's boxes (per-stage bounds when set).
+ * With no bound active this is the exact derivative of the solution; with strict complementarity it tends to the
+ * active-set derivative.  An instance whose last status is not BNMPC_SUCCESS, or that has no multipliers yet, gets NaN rows.
+ * Computed in the handle's precision, FP64 in and out.  One kernel launch per call; the handle's state (iterate,
+ * multipliers, statistics, yref source) is not changed.  on_device: 0 = host buffers, returns with the results in host
+ * memory (staged through handle-owned device memory, allocated on first use, counted by bnmpc_workspace_bytes); 1 = device
+ * buffers, asynchronous on the handle's stream.
+ * d x_k / d x0 and d u_k / d x0 at the stored solution, stages 0 .. stages-1 (1 <= stages <= N+1, else BNMPC_E_ARG):
+ * sens_x [batch][stages][nx][nx], sens_u [batch][min(stages, N)][nu][nx]; either may be NULL.  sens_x[0] = I. */
+int bnmpc_eval_sens_x0(void* handle, int stages, double* sens_x, double* sens_u, int on_device);
+/* The adjoint (vector-Jacobian product) of the same derivative, one solve with the KKT matrix for any seed:
+ * seed_x [batch][N+1][nx], seed_u [batch][N][nu] (NULL = zero, not both: BNMPC_E_ARG); grad_x0 [batch][nx] =
+ * sum_k (d x_k / d x0)' seed_x[k] + (d u_k / d x0)' seed_u[k], grad_yref [batch][N*ny + ny_e] (bnmpc_set_yref_all layout)
+ * the same with respect to the cost reference (0 for the x-part of stage 0: x_0 is fixed by x0); either output may be NULL. */
+int bnmpc_eval_adjoint_sens(void* handle, const double* seed_x, const double* seed_u, double* grad_x0, double* grad_yref, int on_device);
 /* ocp_solver.get_stats / status: int32 [batch] */
 int bnmpc_get_stats(void* handle, int which, int32_t* out, int on_device);
 
