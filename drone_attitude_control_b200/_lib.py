@@ -76,6 +76,8 @@ def lib():
         'bnmpc_step_for_x0': (C.c_int, [vp, dp, dp, dp, dp, dp, vp, dp, C.c_int]),
         'bnmpc_eval_sens_x0': (C.c_int, [vp, C.c_int, dp, dp, C.c_int]),
         'bnmpc_eval_adjoint_sens': (C.c_int, [vp, dp, dp, dp, dp, C.c_int]),
+        'bnmpc_eval_sens_p': (C.c_int, [vp, C.c_int, dp, dp, C.c_int]),
+        'bnmpc_eval_adjoint_sens_p': (C.c_int, [vp, dp, dp, dp, dp, dp, C.c_int]),
         'bnmpc_closed_loop_init': (C.c_int, [vp, dp, dp, dp]),
         'bnmpc_closed_loop_run': (C.c_int, [vp, C.POINTER(ClosedLoopArgs)]),
         'bnmpc_closed_loop_state': (C.c_int, [vp, dp, dp, dp, dp]),

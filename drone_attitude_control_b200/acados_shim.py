@@ -7,6 +7,7 @@ The reference drives acados through `acados_template.AcadosOcpSolver` / `AcadosS
     set(stage, field, value)   get(stage, field)   solve() -> status   get_stats(name)   print_statistics()
     solve_for_x0(x0_bar)       get_cost()          reset()
     eval_solution_sensitivity()             eval_adjoint_solution_sensitivity(seed_x, seed_u)
+    eval_param_sensitivity()                eval_adjoint_param_sensitivity(seed_x, seed_u)
 
 `value` is a `[batch, dim]` tensor (CUDA or CPU) or numpy array; with batch == 1 a plain `(dim,)` numpy vector is
 accepted and `get` returns one, so the reference's `follow_trajectory` runs against this class unchanged apart from the
@@ -288,7 +289,8 @@ class BatchedAcadosOcpSolver:
         (default N + 1): returns (sens_x [batch, stages, nx, nx], sens_u [batch, min(stages, N), nu, nx]) - torch tensors on
         the solver's device, or numpy without the batch dimension when batch == 1, as get() does.  sens_u[:, 0] is the
         feedback gain of u0.  Rows of an instance whose last solve did not succeed are NaN.  Only 'initial_state' is
-        supported (sensitivities with respect to the parameters p are not)."""
+        supported here; the sensitivities with respect to the stage-wise model parameters p = (mass, g) are
+        eval_param_sensitivity (acados' 'p_global' is a different object)."""
         if with_respect_to != 'initial_state':
             raise ValueError(f"with_respect_to={with_respect_to!r}: only 'initial_state' is supported")
         stages = self.N + 1 if stages is None else int(stages)
@@ -315,6 +317,14 @@ class BatchedAcadosOcpSolver:
 
     def adjoint_device(self, seed_x=None, seed_u=None):
         """eval_adjoint_solution_sensitivity with device tensors in and out, asynchronous on the solver's stream."""
+        return self._adjoint(seed_x, seed_u, False)
+
+    def _adjoint_device_p(self, seed_x=None, seed_u=None):
+        """(grad_x0, grad_yref, grad_p) as device tensors from one bnmpc_eval_adjoint_sens_p call, asynchronous on the
+        solver's stream (autograd.solve_u0 with p)."""
+        return self._adjoint(seed_x, seed_u, True)
+
+    def _adjoint(self, seed_x, seed_u, with_p):
         sx = self._seed(seed_x, (self.batch, self.N + 1, self.nx))
         su = self._seed(seed_u, (self.batch, self.N, self.nu))
         if sx is None and su is None:
@@ -322,9 +332,13 @@ class BatchedAcadosOcpSolver:
         gx = torch.empty((self.batch, self.nx), dtype=torch.float64, device=self.device)
         gy = torch.empty((self.batch, self.N * self.ny + self.ny_e), dtype=torch.float64, device=self.device)
         ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
-        check(lib().bnmpc_eval_adjoint_sens(self._h, ptr(sx), ptr(su), ptr(gx), ptr(gy), 1))
         self._keep = (sx, su)
-        return gx, gy
+        if not with_p:
+            check(lib().bnmpc_eval_adjoint_sens(self._h, ptr(sx), ptr(su), ptr(gx), ptr(gy), 1))
+            return gx, gy
+        gp = torch.empty((self.batch, self.np_), dtype=torch.float64, device=self.device)
+        check(lib().bnmpc_eval_adjoint_sens_p(self._h, ptr(sx), ptr(su), ptr(gx), ptr(gy), ptr(gp), 1))
+        return gx, gy, gp
 
     def eval_adjoint_solution_sensitivity(self, seed_x=None, seed_u=None):
         """Adjoint of eval_solution_sensitivity (bnmpc_eval_adjoint_sens): seed_x [batch, N+1, nx], seed_u [batch, N, nu]
@@ -336,6 +350,34 @@ class BatchedAcadosOcpSolver:
             gx, gy = gx.cpu().numpy(), gy.cpu().numpy()
             return (gx[0], gy[0]) if self.batch == 1 else (gx, gy)
         return gx, gy
+
+    # -- sensitivities with respect to the model parameters p = (mass, g) (set(0, 'p', ..); models force, jerk, force_dense) --
+    def eval_param_sensitivity(self, stages=None):
+        """d x_k / d p and d u_k / d p at the solution of the last solve (bnmpc_eval_sens_p), p = (mass, g) of each drone's
+        controller model, stages 0 .. stages-1 (default N + 1): returns (sens_x [batch, stages, nx, np],
+        sens_u [batch, min(stages, N), nu, np]) with the conventions of eval_solution_sensitivity.  sens_x[:, 0] = 0 (x_0 is
+        fixed by x0); sens_u[:, 0, :, 0] is how u0 changes per unit of mass estimate."""
+        stages = self.N + 1 if stages is None else int(stages)
+        if not 1 <= stages <= self.N + 1:
+            raise ValueError(f'stages must be within 1 .. {self.N + 1}, got {stages}')
+        shapes = ((self.batch, stages, self.nx, self.np_), (self.batch, min(stages, self.N), self.nu, self.np_))
+        if self.numpy_io:
+            sx, su = np.empty(shapes[0]), np.empty(shapes[1])
+            check(lib().bnmpc_eval_sens_p(self._h, stages, C.c_void_p(sx.ctypes.data), C.c_void_p(su.ctypes.data), 0))
+            return (sx[0], su[0]) if self.batch == 1 else (sx, su)
+        sx, su = (torch.empty(sh, dtype=torch.float64, device=self.device) for sh in shapes)
+        check(lib().bnmpc_eval_sens_p(self._h, stages, C.c_void_p(sx.data_ptr()), C.c_void_p(su.data_ptr()), 1))
+        return sx, su
+
+    def eval_adjoint_param_sensitivity(self, seed_x=None, seed_u=None):
+        """Adjoint of eval_param_sensitivity (bnmpc_eval_adjoint_sens_p): seed_x [batch, N+1, nx], seed_u [batch, N, nu]
+        (None = 0, not both) -> grad_p [batch, np] = sum over the stages of the sensitivities' transposes times the seeds.
+        One linear solve per drone whatever the seed.  Output types as for eval_solution_sensitivity."""
+        _, _, gp = self._adjoint(seed_x, seed_u, True)
+        if self.numpy_io:
+            gp = gp.cpu().numpy()
+            return gp[0] if self.batch == 1 else gp
+        return gp
 
     def reset(self):
         check(lib().bnmpc_reset(self._h))

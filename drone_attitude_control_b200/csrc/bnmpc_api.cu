@@ -908,31 +908,62 @@ int bnmpc_eval_sens_x0(void* handle, int stages, double* sens_x, double* sens_u,
     return 0;
 }
 
-int bnmpc_eval_adjoint_sens(void* handle, const double* seed_x, const double* seed_u, double* grad_x0, double* grad_yref, int on_device) {
+int bnmpc_eval_sens_p(void* handle, int stages, double* sens_x, double* sens_u, int on_device) {
+    Handle* h = (Handle*)handle;
+    if (!h) return fail(BNMPC_E_ARG, "NULL handle");
+    if (!h->ops->sens) return fail(BNMPC_E_UNSUPPORTED, "solution sensitivities need the exact Hessian of the Lagrangian: models FORCE, JERK and FORCE_DENSE only");
+    const int N = h->cfg.horizon;
+    if (stages < 1 || stages > N + 1) return fail(BNMPC_E_ARG, "stages must be within 1 .. N+1");
+    if (on_device != 0 && on_device != 1) return fail(BNMPC_E_ARG, "on_device must be 0 or 1");
+    if (use_device(h)) return BNMPC_E_CUDA;
+    const size_t B = h->batch, nx = h->ops->nx, nu = h->ops->nu, np = h->ops->np;
+    const size_t nsx = sens_x ? B * stages * nx * np : 0, nsu = sens_u ? B * (stages < N ? stages : N) * nu * np : 0;
+    SensArgs a{stages, sens_x, sens_u, nullptr, nullptr, nullptr, nullptr, nullptr};
+    double* d = nullptr;
+    if (!on_device) {
+        if (int rc = sens_staging(h, nsx + nsu, &d)) return rc;
+        a.sens_x = sens_x ? d : nullptr; a.sens_u = sens_u ? d + nsx : nullptr;
+    }
+    if (int rc = launch_sens(h, a, 2)) return rc;
+    if (on_device) return 0;
+    if (sens_x) CK(cudaMemcpyAsync(sens_x, d, nsx * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (sens_u) CK(cudaMemcpyAsync(sens_u, d + nsx, nsu * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+int bnmpc_eval_adjoint_sens_p(void* handle, const double* seed_x, const double* seed_u, double* grad_x0, double* grad_yref,
+                              double* grad_p, int on_device) {
     Handle* h = (Handle*)handle;
     if (!h) return fail(BNMPC_E_ARG, "NULL handle");
     if (!h->ops->sens) return fail(BNMPC_E_UNSUPPORTED, "solution sensitivities need the exact Hessian of the Lagrangian: models FORCE, JERK and FORCE_DENSE only");
     if (!seed_x && !seed_u) return fail(BNMPC_E_ARG, "seed_x and seed_u are both NULL");
     if (on_device != 0 && on_device != 1) return fail(BNMPC_E_ARG, "on_device must be 0 or 1");
     if (use_device(h)) return BNMPC_E_CUDA;
-    const size_t B = h->batch, nx = h->ops->nx, nu = h->ops->nu, N = h->cfg.horizon;
+    const size_t B = h->batch, nx = h->ops->nx, nu = h->ops->nu, N = h->cfg.horizon, np = h->ops->np;
     const size_t nsx = seed_x ? B * (N + 1) * nx : 0, nsu = seed_u ? B * N * nu : 0;
-    const size_t ngx = grad_x0 ? B * nx : 0, ngy = grad_yref ? B * (N * (nx + nu) + nx) : 0;
-    SensArgs a{0, nullptr, nullptr, seed_x, seed_u, grad_x0, grad_yref};
+    const size_t ngx = grad_x0 ? B * nx : 0, ngy = grad_yref ? B * (N * (nx + nu) + nx) : 0, ngp = grad_p ? B * np : 0;
+    SensArgs a{0, nullptr, nullptr, seed_x, seed_u, grad_x0, grad_yref, grad_p};
     double* d = nullptr;
-    if (!on_device) {       // one staging area: seed_x | seed_u | grad_x0 | grad_yref
-        if (int rc = sens_staging(h, nsx + nsu + ngx + ngy, &d)) return rc;
+    if (!on_device) {       // one staging area: seed_x | seed_u | grad_x0 | grad_yref | grad_p
+        if (int rc = sens_staging(h, nsx + nsu + ngx + ngy + ngp, &d)) return rc;
         if (seed_x) CK(cudaMemcpyAsync(d, seed_x, nsx * sizeof(double), cudaMemcpyHostToDevice, h->stream));
         if (seed_u) CK(cudaMemcpyAsync(d + nsx, seed_u, nsu * sizeof(double), cudaMemcpyHostToDevice, h->stream));
         a.seed_x = seed_x ? d : nullptr; a.seed_u = seed_u ? d + nsx : nullptr;
         a.grad_x0 = grad_x0 ? d + nsx + nsu : nullptr; a.grad_yref = grad_yref ? d + nsx + nsu + ngx : nullptr;
+        a.grad_p = grad_p ? d + nsx + nsu + ngx + ngy : nullptr;
     }
-    if (int rc = launch_sens(h, a, 1)) return rc;
+    if (int rc = launch_sens(h, a, grad_p ? 3 : 1)) return rc;
     if (on_device) return 0;
     if (grad_x0) CK(cudaMemcpyAsync(grad_x0, a.grad_x0, ngx * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     if (grad_yref) CK(cudaMemcpyAsync(grad_yref, a.grad_yref, ngy * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (grad_p) CK(cudaMemcpyAsync(grad_p, a.grad_p, ngp * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return 0;
+}
+
+int bnmpc_eval_adjoint_sens(void* handle, const double* seed_x, const double* seed_u, double* grad_x0, double* grad_yref, int on_device) {
+    return bnmpc_eval_adjoint_sens_p(handle, seed_x, seed_u, grad_x0, grad_yref, nullptr, on_device);
 }
 
 int bnmpc_step_for_x0(void* handle, const double* x0, const double* eps, const double* p_plant, double* u0, double* u_plant,

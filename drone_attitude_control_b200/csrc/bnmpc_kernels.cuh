@@ -65,8 +65,9 @@ struct ModelOps {
     // warps per CTA and warps per instance (wpg; instances in flight per SM = warps / wpg), warps = 0: does not fit
     cudaError_t (*cta_shape)(int N, int* warps, int* wpg);
     long (*loop_static_bytes)(int wpg);                             // static shared memory of the closed-loop kernel (-1: none)
-    // solution sensitivities at the stored solutions, mode 0: d(x_k, u_k) / d x0, 1: adjoint (bnmpc_eval_sens_x0 /
-    // bnmpc_eval_adjoint_sens); nullptr for the models whose Gauss-Newton Hessian is not the Lagrangian's (THRUST, ATT)
+    // solution sensitivities at the stored solutions, mode 0: d(x_k, u_k) / d x0, 1: adjoint, 2: d(x_k, u_k) / d p,
+    // 3: adjoint with grad_p (bnmpc_eval_sens_x0 / bnmpc_eval_adjoint_sens_p / bnmpc_eval_sens_p); nullptr for the models
+    // whose Gauss-Newton Hessian is not the Lagrangian's (THRUST, ATT)
     cudaError_t (*sens)(const GsAny&, const Opts&, const SensArgs&, int mode, int ctas, int warps, int* queue, cudaStream_t);
 };
 
@@ -297,7 +298,8 @@ k_solve(const __grid_constant__ Gs<T> gs, const __grid_constant__ Opts o, const 
     tmem_free_cta(tbase, tmem_cols);
 }
 
-// Solution sensitivities at the stored solutions, MODE 0: forward in x0 (api_sens_x0), 1: adjoint (api_sens_adj).  The
+// Solution sensitivities at the stored solutions, MODE 0: forward in x0 (api_sens_x0), 1: adjoint (api_sens_adj), 2: forward
+// in p (api_sens_p), 3: adjoint with the gradient in p as well.  The
 // launch shape, work queue and shared-memory layout of k_solve, with the per-stage-bound lookup compiled in.  The passes
 // involved (factorisation, Newton solve) keep nothing in the lane-private record, so the kernel allocates no tensor memory.
 template <class M, class T, int MODE>
@@ -308,7 +310,9 @@ k_sens(const __grid_constant__ Gs<T> gs, const __grid_constant__ Opts o, const _
     Solver<M, T, WarpGroup<32>, TmemPriv<M, T, true>> sv(nullptr, warp_smem_off(o.smem_stride), o, g, ps);
     for (int inst = next_instance(queue, nullptr, gs.B); inst < gs.B; inst = next_instance(queue, nullptr, gs.B)) {
         if constexpr (MODE == 0) api_sens_x0<M, T>(sv, inst, gs, a);
-        else api_sens_adj<M, T>(sv, inst, gs, a);
+        else if constexpr (MODE == 1) api_sens_adj<M, T>(sv, inst, gs, a);
+        else if constexpr (MODE == 2) api_sens_p<M, T>(sv, inst, gs, a);
+        else api_sens_adj<M, T, true>(sv, inst, gs, a);
     }
 }
 
@@ -477,6 +481,10 @@ struct OpsImpl {
             if (e != cudaSuccess) return e;
             e = prep(k_sens<M, T, 1>, 0);
             if (e != cudaSuccess) return e;
+            e = prep(k_sens<M, T, 2>, 0);
+            if (e != cudaSuccess) return e;
+            e = prep(k_sens<M, T, 3>, 0);
+            if (e != cudaSuccess) return e;
         }
         int dev = 0, optin = 0;
         e = cudaGetDevice(&dev);
@@ -549,7 +557,9 @@ struct OpsImpl {
         Opts o = o_;
         o.smem_stride = (int)(smem_bytes(o.N) / sizeof(T));
         if (mode == 0) k_sens<M, T, 0><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, sa, queue);
-        else k_sens<M, T, 1><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, sa, queue);
+        else if (mode == 1) k_sens<M, T, 1><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, sa, queue);
+        else if (mode == 2) k_sens<M, T, 2><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, sa, queue);
+        else k_sens<M, T, 3><<<ctas, 32 * warps, smem_bytes(o.N) * warps, st>>>(gs_cast<T>(a), o, sa, queue);
         return cudaGetLastError();
         }
     }

@@ -294,13 +294,16 @@ BN_HD void api_solve(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs, const A
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// solution sensitivities at the stored solutions (bnmpc_eval_sens_x0 / bnmpc_eval_adjoint_sens), FP64 in and out
+// solution sensitivities at the stored solutions (bnmpc_eval_sens_x0 / bnmpc_eval_sens_p / bnmpc_eval_adjoint_sens_p),
+// FP64 in and out
 // ---------------------------------------------------------------------------------------------------------------------
 struct SensArgs {
     int stages;                     // forward: stages 0 .. stages-1 of sens_x, 0 .. min(stages, N)-1 of sens_u
     double *sens_x, *sens_u;        // [B][stages][NX][NX] = d x_k / d x0, [B][min(stages, N)][NU][NX] = d u_k / d x0, or NULL
+                                    // (forward in p: [B][stages][NX][NP], [B][min(stages, N)][NU][NP])
     const double *seed_x, *seed_u;  // adjoint: [B][N+1][NX], [B][N][NU], NULL = 0
     double *grad_x0, *grad_yref;    // [B][NX], [B][N*(NX+NU) + NX] (the bnmpc_set_yref_all layout), or NULL
+    double* grad_p;                 // adjoint: [B][NP] (p = (mass, g)), or NULL
 };
 
 // Binds the instance and factorises its KKT matrix (Solver::sens_factor).  false: the last solve did not succeed or left no
@@ -374,21 +377,130 @@ BN_HD void api_sens_x0(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs, const
     }
 }
 
+// Multiplier step of stage k of the step left by Solver::sens_solve, from item sb1 = (k + 1, b):
+// dpi_k = p_{k+1} + P_{k+1} dx_{k+1} (the multiplier step of Solver::qp_update)
+template <class M, class T, class G, class PS>
+BN_HD void sens_dpi(const Solver<M, T, G, PS>& sv, int sb1, T* dpi) {
+    using SL = typename Solver<M, T, G, PS>::SL;
+    constexpr int n = M::NXB, m = M::NUB;
+#pragma unroll
+    for (int r = 0; r < n; r++) {
+        T d = sv.S(SL::GV + m + r, sb1);
+#pragma unroll
+        for (int l = 0; l < n; l++) d += sv.S(SL::P + sv.pidx(r, l), sb1) * sv.S(SL::DZA + m + l, sb1);
+        dpi[r] = d;
+    }
+}
+
+// The derivative in p_j of the KKT residual of stage k < N, block b, at the stored solution (V: iterate, PI: multipliers of
+// the dynamics, instance bases of Gs): dc = d phi_k / d p_j (the dynamics part) and dr = (d B_k / d p_j)' pi_k (u-part),
+// (d A_k / d p_j)' pi_k (x-part, 0 at stage 0: x_0 is not a variable).  The cost and the bounds do not depend on p.  The
+// three derivatives are the tangents of one pass of the solver's own integrator (rk_dispatch, the scheme of erk_stages,
+// with sensitivities) in dual numbers with p_j seeded: exact derivatives of the code that produced phi, A and B.
+template <class M, class T, class G, class PS>
+BN_HD void sens_rhs_p(const Solver<M, T, G, PS>& sv, const T* V, const T* PI, int k, int b, int j, T* dc, T* dr) {
+    using D = Dual<T>;
+    constexpr int n = M::NXB, m = M::NUB, NX = M::NX, NU = M::NU, NP = M::NP, SG = NX + NU;
+    D p[NP], x[n], u[m], xn[n], A[n * n], B[n * m];
+#pragma unroll
+    for (int i = 0; i < NP; i++) p[i] = D(sv.par[i], i == j ? T(1) : T(0));
+#pragma unroll
+    for (int r = 0; r < n; r++) x[r] = D(V[k * SG + NU + M::xg(b, r)], T(0));
+#pragma unroll
+    for (int c = 0; c < m; c++) u[c] = D(V[k * SG + M::ug(b, c)], T(0));
+    const BlkFn<M, D> fn{b, p};
+    rk_dispatch<n, m, true>(sv.o.erk_stages, fn, x, u, D(T(sv.o.dt), T(0)), xn, A, B);
+    T pi[n];
+#pragma unroll
+    for (int r = 0; r < n; r++) { pi[r] = PI[k * NX + M::xg(b, r)]; dc[r] = xn[r].d; }
+#pragma unroll
+    for (int c = 0; c < m; c++) {
+        T acc = T(0);
+#pragma unroll
+        for (int r = 0; r < n; r++) acc += B[r * m + c].d * pi[r];
+        dr[c] = acc;
+    }
+#pragma unroll
+    for (int c = 0; c < n; c++) {
+        T acc = T(0);
+        if (k >= 1) {
+#pragma unroll
+            for (int r = 0; r < n; r++) acc += A[r * n + c].d * pi[r];
+        }
+        dr[m + c] = acc;
+    }
+}
+
+// Forward in p: d(z, pi) / d p_j = -K^{-1} [dr_j; dc_j] (sens_rhs_p), so direction j is one Newton solve with GV = dr_j and
+// RB = dc_j; its step is column j of d(x_k, u_k) / d p.  sens_x[0] = 0 (x_0 is fixed by x0).  One factorisation, NP solves.
+template <class M, class T, class G, class PS>
+BN_HD void api_sens_p(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs, const SensArgs& a) {
+    using SL = typename Solver<M, T, G, PS>::SL;
+    constexpr int n = M::NXB, m = M::NUB, s = n + m, NBLK = M::NBLK, NX = M::NX, NU = M::NU, NP = M::NP, SG = NX + NU;
+    const int N = sv.N, ns = a.stages, nsu = a.stages < N ? a.stages : N;
+    double* sx = a.sens_x ? a.sens_x + (size_t)inst * ns * NX * NP : nullptr;
+    double* su = a.sens_u ? a.sens_u + (size_t)inst * nsu * NU * NP : nullptr;
+    if (!sens_begin(sv, inst, gs)) {
+        nan_fill(sv.g, sx, (size_t)ns * NX * NP);
+        nan_fill(sv.g, su, (size_t)nsu * NU * NP);
+        sv.g.sync();
+        return;
+    }
+    const T* V = gs.V + (size_t)inst * (N + 1) * SG;
+    const T* PI = gs.PI + (size_t)inst * N * NX;
+    for (int j = 0; j < NP; j++) {
+        for (int sb = sv.g.lane; sb < sv.NSB; sb += G::L) {
+            const int k = sb / NBLK, b = sb % NBLK;
+            sv.use_block(b);
+            T dc[n], dr[s];
+#pragma unroll
+            for (int v = 0; v < s; v++) dr[v] = T(0);
+            if (k < N) {
+                sens_rhs_p(sv, V, PI, k, b, j, dc, dr);
+#pragma unroll
+                for (int r = 0; r < n; r++) sv.S(SL::RB + r, sb) = dc[r];
+            }
+#pragma unroll
+            for (int v = 0; v < s; v++) sv.S(SL::GV + v, sb) = dr[v];
+        }
+        sv.g.sync();
+        sv.sens_solve(ns > 2);
+        for (int sb = sv.g.lane; sb < sv.NSB; sb += G::L) {
+            const int k = sb / NBLK, b = sb % NBLK;
+            if (sx && k < ns) {
+#pragma unroll
+                for (int r = 0; r < n; r++)
+                    sx[((size_t)k * NX + M::xg(b, r)) * NP + j] = k == 0 ? 0.0 : double(sv.S(SL::DZA + m + r, sb));
+            }
+            if (su && k < nsu) {
+#pragma unroll
+                for (int c = 0; c < m; c++) su[((size_t)k * NU + M::ug(b, c)) * NP + j] = double(sv.S(SL::DZA + c, sb));
+            }
+        }
+        sv.g.sync();
+    }
+}
+
 // Adjoint: the KKT matrix is symmetric, so the Newton solve with the seed as gradient (RB = 0) gives the vector-Jacobian
 // products.  With that step (dz, dpi): grad_x0 = seed_x[0] + A_0' dpi_0, and since the cost gradient depends on yref through
 // -dt W (stages < N) / -W_e (stage N), grad_yref = -dt W dz / -W_e dz (0 for the x-part of stage 0: x_0 is not a variable).
-template <class M, class T, class G, class PS>
+// WITH_P (bnmpc_eval_adjoint_sens_p with grad_p): grad_p_j = sum over the stages k < N of dr_j . dz_k + dc_j . dpi_k
+// (sens_rhs_p).  It needs dpi_k, hence dx_k, at every stage, so the forward scan runs whenever grad_p or grad_yref is asked
+// for.  (A separate instantiation: the dual-number integrator would otherwise weigh on the adjoint without grad_p.)
+template <class M, class T, bool WITH_P = false, class G, class PS>
 BN_HD void api_sens_adj(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs, const SensArgs& a) {
     using SL = typename Solver<M, T, G, PS>::SL;
-    constexpr int n = M::NXB, m = M::NUB, s = n + m, NBLK = M::NBLK, NX = M::NX, NU = M::NU, ny = NX + NU;
+    constexpr int n = M::NXB, m = M::NUB, s = n + m, NBLK = M::NBLK, NX = M::NX, NU = M::NU, ny = NX + NU, NP = M::NP;
     const int N = sv.N;
     const double* sdx = a.seed_x ? a.seed_x + (size_t)inst * (N + 1) * NX : nullptr;
     const double* sdu = a.seed_u ? a.seed_u + (size_t)inst * N * NU : nullptr;
     double* gx = a.grad_x0 ? a.grad_x0 + (size_t)inst * NX : nullptr;
     double* gy = a.grad_yref ? a.grad_yref + (size_t)inst * (N * ny + NX) : nullptr;
+    double* gp = WITH_P && a.grad_p ? a.grad_p + (size_t)inst * NP : nullptr;
     if (!sens_begin(sv, inst, gs)) {
         nan_fill(sv.g, gx, NX);
         nan_fill(sv.g, gy, (size_t)N * ny + NX);
+        if constexpr (WITH_P) nan_fill(sv.g, gp, NP);
         sv.g.sync();
         return;
     }
@@ -409,19 +521,12 @@ BN_HD void api_sens_adj(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs, cons
         }
     }
     sv.g.sync();
-    sv.sens_solve(gy != nullptr);
+    sv.sens_solve(gy != nullptr || (WITH_P && gp != nullptr));
     if (gx) {
         for (int b = sv.g.lane; b < NBLK; b += G::L) {
             sv.use_block(b);
-            const int sb1 = NBLK + b;
-            T dpi[n];       // dpi_0 = p_1 + P_1 dx_1 (the multiplier step of Solver::qp_update)
-#pragma unroll
-            for (int r = 0; r < n; r++) {
-                T d = sv.S(SL::GV + m + r, sb1);
-#pragma unroll
-                for (int l = 0; l < n; l++) d += sv.S(SL::P + sv.pidx(r, l), sb1) * sv.S(SL::DZA + m + l, sb1);
-                dpi[r] = d;
-            }
+            T dpi[n];
+            sens_dpi(sv, NBLK + b, dpi);
 #pragma unroll
             for (int c = 0; c < n; c++) {
                 T acc = sdx ? T(sdx[M::xg(b, c)]) : T(0);
@@ -442,6 +547,35 @@ BN_HD void api_sens_adj(Solver<M, T, G, PS>& sv, int inst, const Gs<T>& gs, cons
                 const T h = k < N ? sv.Hd[v] : sv.He[v - m];
                 gy[e] = sv.has(k, v) ? double(-h * sv.S(SL::DZA + v, sb)) : 0.0;
             }
+        }
+    }
+    if constexpr (WITH_P) {
+        const T* V = gs.V + (size_t)inst * (N + 1) * (NX + NU);
+        const T* PI = gs.PI + (size_t)inst * N * NX;
+        T acc[NP];
+#pragma unroll
+        for (int j = 0; j < NP; j++) acc[j] = T(0);
+        for (int sb = sv.g.lane; sb < sv.NSB - NBLK; sb += G::L) {
+            const int k = sb / NBLK, b = sb % NBLK;
+            sv.use_block(b);
+            T dpi[n];
+            sens_dpi(sv, sb + NBLK, dpi);
+#pragma unroll
+            for (int j = 0; j < NP; j++) {
+                T dc[n], dr[s];
+                sens_rhs_p(sv, V, PI, k, b, j, dc, dr);
+                T c = T(0);
+#pragma unroll
+                for (int r = 0; r < n; r++) c += dc[r] * dpi[r];
+#pragma unroll
+                for (int v = 0; v < s; v++) if (sv.has(k, v)) c += dr[v] * sv.S(SL::DZA + v, sb);
+                acc[j] += c;
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < NP; j++) {
+            const T t = sv.g.sum(acc[j]);
+            if (sv.g.lane == 0) gp[j] = double(t);
         }
     }
     sv.g.sync();

@@ -198,8 +198,21 @@ int bnmpc_eval_sens_x0(void* handle, int stages, double* sens_x, double* sens_u,
 /* The adjoint (vector-Jacobian product) of the same derivative, one solve with the KKT matrix for any seed:
  * seed_x [batch][N+1][nx], seed_u [batch][N][nu] (NULL = zero, not both: BNMPC_E_ARG); grad_x0 [batch][nx] =
  * sum_k (d x_k / d x0)' seed_x[k] + (d u_k / d x0)' seed_u[k], grad_yref [batch][N*ny + ny_e] (bnmpc_set_yref_all layout)
- * the same with respect to the cost reference (0 for the x-part of stage 0: x_0 is fixed by x0); either output may be NULL. */
+ * the same with respect to the cost reference (0 for the x-part of stage 0: x_0 is fixed by x0); either output may be NULL.
+ * This is bnmpc_eval_adjoint_sens_p with grad_p = NULL. */
 int bnmpc_eval_adjoint_sens(void* handle, const double* seed_x, const double* seed_u, double* grad_x0, double* grad_yref, int on_device);
+/* d x_k / d p and d u_k / d p at the stored solution, p = (mass, g) of the controller model (BNMPC_F_P, np = 2), stages
+ * 0 .. stages-1 (1 <= stages <= N+1, else BNMPC_E_ARG): sens_x [batch][stages][nx][np], sens_u [batch][min(stages, N)][nu][np];
+ * either may be NULL.  sens_x[0] = 0 (x_0 is fixed by x0).  With the same KKT matrix and c_k = phi_k(x_k, u_k; p) - x_{k+1}:
+ * d(z, pi) / d p_j = -K^{-1} [dR_j; dc_j], dc_j = d phi_k / d p_j, dR_j = (d B_k / d p_j)' pi_k (u-part),
+ * (d A_k / d p_j)' pi_k (x-part, stages >= 1), where phi_k, A_k, B_k are the configured integrator (erk_stages) and its
+ * sensitivities, differentiated exactly.  One factorisation and np solves per instance. */
+int bnmpc_eval_sens_p(void* handle, int stages, double* sens_x, double* sens_u, int on_device);
+/* bnmpc_eval_adjoint_sens plus grad_p [batch][np] = sum_k (d x_k / d p)' seed_x[k] + (d u_k / d p)' seed_u[k], all from one
+ * solve with the KKT matrix; any output may be NULL.  With grad_p = NULL this is bnmpc_eval_adjoint_sens, bit for bit; with
+ * grad_p, grad_x0 and grad_yref agree with it to rounding (the evaluation of grad_p is a separate kernel instantiation). */
+int bnmpc_eval_adjoint_sens_p(void* handle, const double* seed_x, const double* seed_u, double* grad_x0, double* grad_yref,
+                              double* grad_p, int on_device);
 /* ocp_solver.get_stats / status: int32 [batch] */
 int bnmpc_get_stats(void* handle, int which, int32_t* out, int on_device);
 

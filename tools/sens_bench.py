@@ -2,7 +2,8 @@
 
 For each case (force model with 4096 drones, jerk model with 16384 drones, FP64, reference horizon N = 30) it times, per
 call: the solve (solve_for_x0_device), bnmpc_eval_sens_x0 with stages = 1 (the feedback gain of u0) and with stages = N + 1,
-and the adjoint with a seed on u0 only.  Each timed solve starts from the solution of the previous one at another x0 (the
+the adjoint with a seed on u0 only, bnmpc_eval_sens_p (p = (mass, g)) with stages = 1 and N + 1, and the adjoint with a seed
+on u0 that also returns grad_p.  Each timed solve starts from the solution of the previous one at another x0 (the
 x0 sets alternate), so that it is a real re-solve, as in a closed loop; its mean QP iterations are recorded.  The
 sensitivities are evaluated at the stored solution, which they leave as it is.  10 warm-up and 50 timed calls, three
 repeats; the card's name and power limit are read in the same run.
@@ -87,9 +88,20 @@ def case(model, B):
     res['sens_x0_stages1_ms'] = timed(lambda: check(lib().bnmpc_eval_sens_x0(sv.handle, 1, p(sx1), p(su1), 1)), st)
     res['sens_x0_stagesN1_ms'] = timed(lambda: check(lib().bnmpc_eval_sens_x0(sv.handle, N + 1, p(sxN), p(suN), 1)), st)
     res['adjoint_seed_u0_ms'] = timed(lambda: check(lib().bnmpc_eval_adjoint_sens(sv.handle, None, p(seed_u), p(gx), p(gy), 1)), st)
+    spx1, spu1 = (torch.empty((B, 1, sv.nx, sv.np_), dtype=torch.float64, device=dev),
+                  torch.empty((B, 1, sv.nu, sv.np_), dtype=torch.float64, device=dev))
+    spxN, spuN = (torch.empty((B, N + 1, sv.nx, sv.np_), dtype=torch.float64, device=dev),
+                  torch.empty((B, N, sv.nu, sv.np_), dtype=torch.float64, device=dev))
+    gp = torch.empty((B, sv.np_), dtype=torch.float64, device=dev)
+    res['sens_p_stages1_ms'] = timed(lambda: check(lib().bnmpc_eval_sens_p(sv.handle, 1, p(spx1), p(spu1), 1)), st)
+    res['sens_p_stagesN1_ms'] = timed(lambda: check(lib().bnmpc_eval_sens_p(sv.handle, N + 1, p(spxN), p(spuN), 1)), st)
+    res['adjoint_p_seed_u0_ms'] = timed(
+        lambda: check(lib().bnmpc_eval_adjoint_sens_p(sv.handle, None, p(seed_u), p(gx), p(gy), p(gp), 1)), st)
     torch.cuda.synchronize()
     res['sens_nan_rows'] = int(torch.isnan(su1).any(-1).any(-1).any(-1).sum())
-    for k in ('sens_x0_stages1_ms', 'sens_x0_stagesN1_ms', 'adjoint_seed_u0_ms'):
+    res['sens_p_nan_rows'] = int(torch.isnan(spu1).any(-1).any(-1).any(-1).sum())
+    for k in ('sens_x0_stages1_ms', 'sens_x0_stagesN1_ms', 'adjoint_seed_u0_ms', 'sens_p_stages1_ms', 'sens_p_stagesN1_ms',
+              'adjoint_p_seed_u0_ms'):
         res[k.replace('_ms', '_over_solve')] = float(np.median(res[k]) / np.median(res['solve_ms']))
     return res
 
